@@ -1,6 +1,6 @@
-"""Generate the committed golden fixtures.  Run in the BUILD container (needs /root/reference):
+"""Generate the committed golden fixtures from a LiveTalking checkout:
 
-    python tests/golden/make_golden.py
+    LTB_REFERENCE=<LiveTalking checkout> python tests/golden/make_golden.py
 
 * w2l_golden.npz   — the UNMODIFIED reference nn.Module (avatars/wav2lip/models/wav2lip_v2.py, imported by file
                      path) run on CPU fp32 with the seeded synthetic weights of oracle.wav2lip_ref.synth_state_dict(0)
@@ -21,6 +21,9 @@
 * lipreal_golden.npz — LipReal.inference_batch + paste_back_frame run from the reference module (a4 + a5 + a6 glue).
 * pe_golden.npz, vae_glue_golden.npz, musereal_golden.npz — the reference's PositionalEncoding, VAE.preprocess_img /
                      decode_latents and MuseReal.inference_batch (third-party networks replaced by recorders / fakes).
+* asr_host_golden.npz — the reference's own BaseASR / WhisperASR / HubertASR queue bookkeeping (extractors replaced by
+                     recorders) on the seeded event sequences of tests/test_plugin_host.py.
+* mt_blend_golden.npz — the reference's own get_image_blending (avatars/musetalk/myutil.py) on a seeded MuseTalk paste-back.
 Every generator is deterministic: re-running this script reproduces the committed files byte for byte.
 """
 import importlib.util
@@ -35,7 +38,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import wav2lip_ref as R  # noqa: E402
 
-REF = "/root/reference"
+REF = os.environ.get("LTB_REFERENCE", "")
 
 
 def load_reference_wav2lip():
@@ -509,7 +512,119 @@ def make_ultralight():
     print("ultralight golden ok", out.shape, float(out.mean()), float(out.std()), pred.dtype)
 
 
+def _audio_records(frames):
+    """AudioFrameData list -> (types, data, userdata as JSON strings)."""
+    import json
+    return (np.asarray([f.type for f in frames], np.int32), np.stack([np.asarray(f.data, np.float32) for f in frames]),
+            np.asarray([json.dumps(f.userdata, sort_keys=True) for f in frames]))
+
+
+def _drain(q):
+    return [q.get() for _ in range(q.qsize())]
+
+
+def make_asr_host():
+    """The reference's OWN BaseASR / WhisperASR / HubertASR (avatars/audio_features/*.py, imported by file path, feature
+    extractors replaced by recorders) on the seeded event sequences of tests/test_plugin_host.py: frames pulled, queues,
+    the PCM context handed to the extractor, the context buffer kept.  Pins the plugin's queue bookkeeping."""
+    sys.path.insert(0, os.path.join(HERE, ".."))
+    import stubs
+    stubs.install()
+    from test_plugin_host import _feed
+
+    def load(name, rel):
+        spec = importlib.util.spec_from_file_location(name, os.path.join(REF, rel))
+        m = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(m)
+        return m
+
+    out = {}
+    base = load("ref_base_asr", "avatars/audio_features/base_asr.py")
+    a = base.BaseASR(stubs.Opt(batch_size=3))                   # test_same_behaviour_as_reference_base_asr
+    _feed(a, 23, np.random.default_rng(5))
+    a.warm_up()
+    out["base_get_type"], out["base_get_data"], out["base_get_ud"] = _audio_records([a.get_audio_frame() for _ in range(8)])
+    out["base_outq"] = np.int64(a.output_queue.qsize())
+    out["base_frames"] = np.stack(a.frames).astype(np.float32)
+
+    af = types.ModuleType("avatars.audio_features")
+    af.__path__ = []
+    sys.modules["avatars.audio_features"] = af
+    sys.modules["avatars.audio_features.base_asr"] = base
+    for name in ("avatars.musetalk", "avatars.musetalk.whisper", "avatars.ultralight"):
+        sys.modules.setdefault(name, types.ModuleType(name))
+    for name in ("avatars.musetalk.whisper.audio2feature", "avatars.ultralight.audio2feature"):
+        sys.modules[name] = types.ModuleType(name)
+        sys.modules[name].Audio2Feature = object
+
+    B = 3                                                       # test_whisper_asr_run_step_bookkeeping_matches_reference
+    whisper = load("ref_whisper_asr", "avatars/audio_features/whisper.py")
+
+    class WhisperRecorder:
+        def __init__(self):
+            self.calls = []
+
+        def audio2feat(self, pcm):
+            self.calls.append(np.asarray(pcm).copy())
+            return np.zeros((1500, 5, 384), np.float32)
+
+    rec = WhisperRecorder()
+    w = whisper.WhisperASR(stubs.Opt(batch_size=B), None, rec)
+    _feed(w, 20 + 2 * B + 2, np.random.default_rng(2))
+    w.warm_up()
+    w.run_step()
+    assert w.feat_queue.qsize() == 1 and len(rec.calls) == 1
+    out["whisper_feat_shape"] = np.asarray([np.asarray(f).shape for f in w.feat_queue.get()], np.int32)
+    out["whisper_pcm"] = rec.calls[0].astype(np.float32)
+    out["whisper_frames"] = np.stack(w.frames).astype(np.float32)
+    out["whisper_out_type"], out["whisper_out_data"], _ = _audio_records(_drain(w.output_queue))
+
+    hubert = load("ref_hubert_asr", "avatars/audio_features/hubert.py")   # test_hubert_asr_run_step_bookkeeping_matches_reference
+
+    class HubertRecorder:
+        def __init__(self):
+            self.calls = []
+
+        def get_hubert_from_16k_speech(self, pcm):
+            self.calls.append(np.asarray(pcm).copy())
+            return np.ones(((len(pcm) - 80) // 320, 1024), np.float32)
+
+    rec = HubertRecorder()
+    h = hubert.HubertASR(stubs.Opt(batch_size=B), None, rec, audio_feat_length=[4, 4])
+    _feed(h, 20 + 2 * B, np.random.default_rng(4))
+    h.warm_up()
+    shapes = []
+    for _step in range(3):
+        h.run_step()
+        shapes.append([np.asarray(f).shape for f in h.feat_queue.get()])
+    out["hubert_feat_shapes"] = np.asarray(shapes, np.int32)
+    out["hubert_pcm"] = np.stack(rec.calls).astype(np.float32)
+    out["hubert_last_is_silence"] = np.bool_(h.last_is_silence)
+    out["hubert_frames"] = np.stack(h.frames).astype(np.float32)
+    out["hubert_out_type"], out["hubert_out_data"], _ = _audio_records(_drain(h.output_queue))
+    np.savez_compressed(os.path.join(HERE, "asr_host_golden.npz"), **out)
+    print("asr host golden ok", {k: v.shape for k, v in out.items()})
+
+
+def make_mt_blend():
+    """The reference's OWN get_image_blending (avatars/musetalk/myutil.py) driven as MuseReal.paste_back_frame does, on the
+    seeded frame / prediction / masks of tests/test_oracle_paste.py::test_musetalk_blend_matches_cv2_and_reference_function."""
+    import cv2
+    sys.path.insert(0, os.path.join(HERE, ".."))
+    from test_oracle_paste import mt_blend_case
+    spec = importlib.util.spec_from_file_location("ref_myutil", os.path.join(REF, "avatars/musetalk/myutil.py"))
+    ref = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(ref)
+    frame, pred, bbox, crop, masks = mt_blend_case()
+    x1, y1, x2, y2 = bbox
+    want = [ref.get_image_blending(frame.copy(), cv2.resize(pred, (x2 - x1, y2 - y1)), bbox, m, crop) for m in masks]
+    np.savez_compressed(os.path.join(HERE, "mt_blend_golden.npz"), want=np.stack(want))
+    print("mt blend golden ok", np.stack(want).shape)
+
+
 if __name__ == "__main__":
+    if not os.path.isfile(os.path.join(REF, "avatars", "base_avatar.py")):
+        sys.exit("set LTB_REFERENCE to a LiveTalking checkout")
     make_w2l()
     make_paste()
     make_mel()
@@ -521,3 +636,5 @@ if __name__ == "__main__":
     make_mel_chain()
     make_musereal()
     make_ultralight()
+    make_asr_host()
+    make_mt_blend()

@@ -4,7 +4,8 @@
 modules injected (the technique of the reference's own tests/test_asr_server.py:57-72 — those three are transport / file
 decoding dependencies that the per-frame path never calls).
 
-Only usable where the reference tree exists (this container); GPU-box tests use ``stubs.ThreeThreadDriver`` instead.
+Used where a LiveTalking checkout is named by the LTB_REFERENCE environment variable; elsewhere ``reference_runtime`` hands out
+the host of tests/stubs.py instead, whose ``BaseAvatar`` runs the same three-thread render loop, so the tests run everywhere.
 Only the swapped module names (reference modules, the three fakes, the plugin modules) are saved and restored, so the
 process-wide stubs other tests install come back afterwards and torch / cv2 stay loaded."""
 from __future__ import annotations
@@ -18,7 +19,7 @@ import types
 
 import numpy as np
 
-REF = os.environ.get("LTB_REFERENCE", "/root/reference")
+REF = os.environ.get("LTB_REFERENCE", "")
 
 _REF_MODULES = ("avatars", "avatars.base_avatar", "avatars.audio_features", "avatars.audio_features.base_asr", "registry", "utils",
                 "utils.image", "utils.logger")
@@ -29,7 +30,7 @@ _PLUGIN_MODULES = ("livetalking_b200.plugin", "livetalking_b200.plugin.base_asr"
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REF, "avatars", "base_avatar.py"))
+    return bool(REF) and os.path.isfile(os.path.join(REF, "avatars", "base_avatar.py"))
 
 
 def _fake_modules():
@@ -49,12 +50,31 @@ def _fake_modules():
     return {"av": av, "resampy": resampy, "soundfile": soundfile}
 
 
+def _namespace(reference: bool):
+    base = sys.modules["avatars.base_avatar"]
+    ns = types.SimpleNamespace(reference=reference, base_avatar=base, registry=importlib.import_module("registry"),
+                               AudioFrameData=base.AudioFrameData, mirror_index=importlib.import_module("utils.image").mirror_index,
+                               plugin_w2l=importlib.import_module("livetalking_b200.plugin.wav2lip_avatar"),
+                               plugin_base_asr=importlib.import_module("livetalking_b200.plugin.base_asr"))
+    ns.load_musetalk = lambda: importlib.import_module("livetalking_b200.plugin.musetalk_avatar")
+    ns.load_ultralight = lambda: importlib.import_module("livetalking_b200.plugin.ultralight_avatar")
+    return ns
+
+
 @contextlib.contextmanager
 def reference_runtime(workdir: str):
-    """-> namespace(base_avatar, registry, plugin_w2l, plugin_mt (lazy), AudioFrameData, mirror_index)."""
-    if not available():
-        raise RuntimeError("reference checkout not present")
+    """-> namespace(reference, base_avatar, registry, plugin_w2l, plugin_base_asr, load_musetalk, load_ultralight,
+    AudioFrameData, mirror_index): the reference's own runtime when available(), else the host of tests/stubs.py."""
     old_cwd = os.getcwd()
+    if not available():
+        import stubs
+        stubs.install()
+        os.chdir(workdir)
+        try:
+            yield _namespace(reference=False)
+        finally:
+            os.chdir(old_cwd)
+        return
     os.chdir(workdir)                              # utils/logger.py opens ./livetalking.log at import
     fakes = _fake_modules()
     managed = tuple(fakes) + _REF_MODULES + _PLUGIN_MODULES
@@ -66,14 +86,7 @@ def reference_runtime(workdir: str):
     try:
         base = importlib.import_module("avatars.base_avatar")
         assert os.path.samefile(base.__file__, os.path.join(REF, "avatars", "base_avatar.py")), "not the reference's module"
-        ns = types.SimpleNamespace(base_avatar=base, registry=importlib.import_module("registry"),
-                                   AudioFrameData=base.AudioFrameData,
-                                   mirror_index=importlib.import_module("utils.image").mirror_index,
-                                   plugin_w2l=importlib.import_module("livetalking_b200.plugin.wav2lip_avatar"),
-                                   plugin_base_asr=importlib.import_module("livetalking_b200.plugin.base_asr"))
-        ns.load_musetalk = lambda: importlib.import_module("livetalking_b200.plugin.musetalk_avatar")
-        ns.load_ultralight = lambda: importlib.import_module("livetalking_b200.plugin.ultralight_avatar")
-        yield ns
+        yield _namespace(reference=True)
     finally:
         sys.path.remove(REF)
         os.chdir(old_cwd)

@@ -44,10 +44,9 @@ def test_mirror_index_and_batch_build():
     assert np.all(b[0, :3, :128] == np.float32(20 / 255.0))
 
 
-def test_musetalk_blend_matches_cv2_and_reference_function():
-    """oracle mt_paste_back vs OpenCV (blendLinear / cvtColor) and, in the build container, vs the reference's own
-    get_image_blending (avatars/musetalk/myutil.py) driven as MuseReal.paste_back_frame does."""
-    cv2 = pytest.importorskip("cv2")
+def mt_blend_case():
+    """Seeded MuseTalk paste-back case: frame, prediction, bbox, crop, [soft mask, noise mask]."""
+    import cv2
     rng = np.random.default_rng(3)
     H, W = 180, 240
     frame = rng.integers(0, 256, (H, W, 3), dtype=np.uint8)
@@ -57,7 +56,17 @@ def test_musetalk_blend_matches_cv2_and_reference_function():
     mh, mw = crop[3] - crop[1], crop[2] - crop[0]
     soft = cv2.GaussianBlur((np.arange(mh)[:, None] > mh // 2).astype(np.float32).repeat(mw, 1) * 255, (0, 0), 7).astype(np.uint8)
     masks = [np.stack([soft] * 3, -1), rng.integers(0, 256, (mh, mw, 3), dtype=np.uint8)]
-    for mask in masks:
+    return frame, pred, bbox, crop, masks
+
+
+def test_musetalk_blend_matches_cv2_and_reference_function(golden_dir):
+    """oracle mt_paste_back vs OpenCV (blendLinear / cvtColor) and vs the output of the reference's own get_image_blending
+    (avatars/musetalk/myutil.py) driven as MuseReal.paste_back_frame does (mt_blend_golden.npz)."""
+    cv2 = pytest.importorskip("cv2")
+    frame, pred, bbox, crop, masks = mt_blend_case()
+    want = np.load(os.path.join(golden_dir, "mt_blend_golden.npz"))["want"]
+    assert want.shape == (len(masks),) + frame.shape
+    for mask, ref_out in zip(masks, want):
         got = P.mt_paste_back(pred, frame, bbox, mask, crop)
         # direct OpenCV composition
         x1, y1, x2, y2 = bbox
@@ -68,11 +77,4 @@ def test_musetalk_blend_matches_cv2_and_reference_function():
         m = (cv2.cvtColor(mask, cv2.COLOR_BGR2GRAY) / 255).astype(np.float32)
         body[ys:ye, xs:xe] = cv2.blendLinear(large, body[ys:ye, xs:xe], m, 1 - m)
         assert np.array_equal(got, body)
-        ref_path = "/root/reference/avatars/musetalk/myutil.py"
-        if os.path.exists(ref_path):
-            import importlib.util
-            spec = importlib.util.spec_from_file_location("ref_myutil", ref_path)
-            ref = importlib.util.module_from_spec(spec)
-            spec.loader.exec_module(ref)
-            want = ref.get_image_blending(frame.copy(), cv2.resize(pred.astype(np.uint8), (x2 - x1, y2 - y1)), bbox, mask, crop)
-            assert np.array_equal(got, want)
+        assert np.array_equal(got, ref_out)

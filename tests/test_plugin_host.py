@@ -1,6 +1,7 @@
-"""CPU: host-side logic of the plugin layer (queues, silence synthesis, warm-up, run_step bookkeeping), and — when the
-reference tree is present (build container) — equivalence with the reference's own BaseASR on the same event sequence."""
-import importlib.util
+"""CPU: host-side logic of the plugin layer (queues, silence synthesis, warm-up, run_step bookkeeping), and equivalence with
+the reference's own BaseASR / WhisperASR / HubertASR on the same event sequences (their results are stored in
+tests/golden/asr_host_golden.npz by tests/golden/make_golden.py::make_asr_host)."""
+import json
 import os
 import sys
 
@@ -19,6 +20,26 @@ def _feed(asr, n, rng):
     for i, c in enumerate(chunks):
         asr.put_audio_frame(c, {"i": i})
     return chunks
+
+
+def _golden():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "asr_host_golden.npz"))
+
+
+def _assert_records(frames, types, data, userdata=None):
+    assert len(frames) == len(types)
+    for k, f in enumerate(frames):
+        assert f.type == types[k] and np.array_equal(np.asarray(f.data, np.float32), data[k])
+        if userdata is not None:
+            assert f.userdata == json.loads(str(userdata[k]))
+
+
+def _assert_frames(frames, want):
+    assert len(frames) == len(want) and all(np.array_equal(x, y) for x, y in zip(frames, want))
+
+
+def _drain(q):
+    return [q.get() for _ in range(q.qsize())]
 
 
 def test_silence_synthesis_and_warm_up():
@@ -50,23 +71,15 @@ def test_custom_audio_stream_has_priority():
     assert f.type == 2 and float(f.data[0]) == 0.25      # base_asr.py:59-62
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/avatars/audio_features/base_asr.py"), reason="reference tree not present")
 def test_same_behaviour_as_reference_base_asr():
-    spec = importlib.util.spec_from_file_location("ref_base_asr", "/root/reference/avatars/audio_features/base_asr.py")
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)                         # imports the stubbed avatars.base_avatar
-    opt = stubs.Opt(batch_size=3)
-    ours, theirs = B.BaseASR(opt), ref.BaseASR(opt)
-    rng1, rng2 = np.random.default_rng(5), np.random.default_rng(5)
-    _feed(ours, 23, rng1)
-    _feed(theirs, 23, rng2)
+    g = _golden()
+    ours = B.BaseASR(stubs.Opt(batch_size=3))
+    _feed(ours, 23, np.random.default_rng(5))
     ours.warm_up()
-    theirs.warm_up()
-    for _ in range(8):                                   # drains speech then synthesises silence
-        a, b = ours.get_audio_frame(), theirs.get_audio_frame()
-        assert a.type == b.type and np.array_equal(a.data, b.data) and a.userdata == b.userdata
-    assert ours.output_queue.qsize() == theirs.output_queue.qsize()
-    assert len(ours.frames) == len(theirs.frames) and all(np.array_equal(x, y) for x, y in zip(ours.frames, theirs.frames))
+    got = [ours.get_audio_frame() for _ in range(8)]     # drains speech then synthesises silence
+    _assert_records(got, g["base_get_type"], g["base_get_data"], g["base_get_ud"])
+    assert ours.output_queue.qsize() == int(g["base_outq"])
+    _assert_frames(ours.frames, g["base_frames"])
 
 
 def test_mel_asr_run_step_bookkeeping_with_fake_session():
@@ -99,8 +112,8 @@ def test_mel_asr_run_step_bookkeeping_with_fake_session():
 
 def test_whisper_asr_run_step_bookkeeping_matches_reference():
     """WhisperASR.run_step (whisper.py:58-76): 2B chunks forwarded, the whole l+r+2B context handed to the feature extractor,
-    one list of B (50, 384) arrays queued, l+r chunks kept.  In the build container the reference's own class runs the same
-    event sequence (its Audio2Feature replaced by a recorder) and every queue / buffer must match."""
+    one list of B (50, 384) arrays queued, l+r chunks kept.  Every queue / buffer must match what the reference's own class
+    recorded on the same event sequence (its Audio2Feature replaced by a recorder)."""
     from livetalking_b200.plugin.whisper_asr import WhisperASR
 
     class FakeFeatures:                                   # stands in for livetalking_b200.whisper.WhisperFeatures
@@ -127,62 +140,18 @@ def test_whisper_asr_run_step_bookkeeping_matches_reference():
     with pytest.raises(RuntimeError):
         WhisperASR(opt, None, None)                       # no engine object -> loud failure, never a CPU fallback
 
-    ref_path = "/root/reference/avatars/audio_features/whisper.py"
-    if not os.path.exists(ref_path):
-        return
-    import types
-    a2f = types.ModuleType("avatars.musetalk.whisper.audio2feature")
-    a2f.Audio2Feature = object
-    for name in ("avatars.musetalk", "avatars.musetalk.whisper"):
-        sys.modules.setdefault(name, types.ModuleType(name))
-    sys.modules["avatars.musetalk.whisper.audio2feature"] = a2f
-    spec = importlib.util.spec_from_file_location("ref_base_asr2", "/root/reference/avatars/audio_features/base_asr.py")
-    ref_base = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref_base)
-    af = types.ModuleType("avatars.audio_features")
-    af.__path__ = []
-    sys.modules["avatars.audio_features"] = af
-    sys.modules["avatars.audio_features.base_asr"] = ref_base
-    spec = importlib.util.spec_from_file_location("ref_whisper_asr", ref_path)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-
-    class Recorder:                                        # the reference's audio_processor: (T, 5, 384) hidden-state stack
-        def __init__(self):
-            self.calls = []
-
-        def audio2feat(self, pcm):
-            self.calls.append(np.asarray(pcm).copy())
-            return np.zeros((1500, 5, 384), np.float32)
-
-    rec = Recorder()
-    theirs = ref.WhisperASR(opt, None, rec)
-    _feed(theirs, 20 + 2 * B + 2, np.random.default_rng(2))
-    theirs.warm_up()
-    theirs.run_step()
-    fake2 = FakeFeatures(B)
-    again = WhisperASR(opt, None, fake2)
-    _feed(again, 20 + 2 * B + 2, np.random.default_rng(2))
-    again.warm_up()
-    again.run_step()
-    assert theirs.feat_queue.qsize() == again.feat_queue.qsize() == 1
-    assert theirs.output_queue.qsize() == again.output_queue.qsize()
-    tf, of = theirs.feat_queue.get(), again.feat_queue.get()
-    assert len(tf) == len(of) == B and tf[0].shape == of[0].shape == (50, 384)
-    assert np.array_equal(rec.calls[0], fake2.calls[0])                                # identical PCM context handed over
-    assert len(theirs.frames) == len(again.frames) and all(np.array_equal(x, y) for x, y in zip(theirs.frames, again.frames))
-    for _ in range(theirs.output_queue.qsize()):
-        a, b = theirs.output_queue.get(), again.output_queue.get()
-        assert a.type == b.type and np.array_equal(a.data, b.data)
-    for k in ("avatars.audio_features", "avatars.audio_features.base_asr", "avatars.musetalk.whisper.audio2feature"):
-        sys.modules.pop(k, None)
+    g = _golden()
+    assert np.array_equal(np.asarray([np.asarray(f).shape for f in feats]), g["whisper_feat_shape"])
+    assert np.array_equal(fake.calls[0], g["whisper_pcm"])                              # identical PCM context handed over
+    _assert_frames(ours.frames, g["whisper_frames"])
+    _assert_records(_drain(ours.output_queue), g["whisper_out_type"], g["whisper_out_data"])
 
 
 def test_hubert_asr_run_step_bookkeeping_matches_reference():
     """HubertASR.run_step (avatars/audio_features/hubert.py:27-51): 2B chunks forwarded, silence tracking over TWO batches (features
     are computed unless this batch and the previous one were all silence), the whole l+r+2B context handed to the extractor, one
-    list of B windows queued, l+r chunks kept.  In the build container the reference's own class runs the same event sequence
-    (speech, then two silent steps) with its Audio2Feature replaced by a recorder; every queue / buffer / flag must match."""
+    list of B windows queued, l+r chunks kept.  Every queue / buffer / flag must match what the reference's own class recorded on
+    the same event sequence (speech, then two silent steps) with its Audio2Feature replaced by a recorder."""
     from livetalking_b200.plugin.hubert_asr import HubertASR
 
     class FakeFeatures:                                   # stands in for livetalking_b200.hubert.HubertFeatures
@@ -213,43 +182,9 @@ def test_hubert_asr_run_step_bookkeeping_matches_reference():
     with pytest.raises(RuntimeError):
         HubertASR(opt, None, None)                        # no engine object -> loud failure, never a CPU fallback
 
-    ref_path = "/root/reference/avatars/audio_features/hubert.py"
-    if not os.path.exists(ref_path):
-        return
-    import types
-    a2f = types.ModuleType("avatars.ultralight.audio2feature")
-    a2f.Audio2Feature = object
-    sys.modules.setdefault("avatars.ultralight", types.ModuleType("avatars.ultralight"))
-    sys.modules["avatars.ultralight.audio2feature"] = a2f
-    spec = importlib.util.spec_from_file_location("ref_base_asr3", "/root/reference/avatars/audio_features/base_asr.py")
-    ref_base = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref_base)
-    af = types.ModuleType("avatars.audio_features")
-    af.__path__ = []
-    sys.modules["avatars.audio_features"] = af
-    sys.modules["avatars.audio_features.base_asr"] = ref_base
-    spec = importlib.util.spec_from_file_location("ref_hubert_asr", ref_path)
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-
-    class Recorder:                                        # the reference's audio_processor
-        def __init__(self):
-            self.calls = []
-
-        def get_hubert_from_16k_speech(self, pcm):
-            self.calls.append(np.asarray(pcm).copy())
-            return np.ones(((len(pcm) - 80) // 320, 1024), np.float32)
-
-    rec = Recorder()
-    theirs = ref.HubertASR(opt, None, rec, audio_feat_length=[4, 4])
-    tshapes = drive(theirs)
-    assert tshapes == shapes
-    assert len(rec.calls) == len(fake.calls) and all(np.array_equal(a, b) for a, b in zip(rec.calls, fake.calls))
-    assert theirs.last_is_silence == ours.last_is_silence
-    assert len(theirs.frames) == len(ours.frames) and all(np.array_equal(x, y) for x, y in zip(theirs.frames, ours.frames))
-    assert theirs.output_queue.qsize() == ours.output_queue.qsize()
-    for _ in range(theirs.output_queue.qsize()):
-        a, b = theirs.output_queue.get(), ours.output_queue.get()
-        assert a.type == b.type and np.array_equal(a.data, b.data)
-    for k in ("avatars.audio_features", "avatars.audio_features.base_asr", "avatars.ultralight.audio2feature", "avatars.ultralight"):
-        sys.modules.pop(k, None)
+    g = _golden()
+    assert np.array_equal(np.asarray(shapes), g["hubert_feat_shapes"])
+    assert len(fake.calls) == len(g["hubert_pcm"]) and all(np.array_equal(a, b) for a, b in zip(fake.calls, g["hubert_pcm"]))
+    assert ours.last_is_silence == bool(g["hubert_last_is_silence"])
+    _assert_frames(ours.frames, g["hubert_frames"])
+    _assert_records(_drain(ours.output_queue), g["hubert_out_type"], g["hubert_out_data"])
