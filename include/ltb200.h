@@ -48,10 +48,18 @@ int ltb_w2l_model_destroy(ltb_w2l_model* m);
 
 /* ---- avatar assets ---------------------------------------------------------------------------------- */
 /* replaces load_avatar(avatar_id), avatars/wav2lip_avatar.py:72-88: face crops (n,256,256,3) u8 BGR, full frames
- * (n,H,W,3) u8 BGR and coords (n,4) int32 = (y1,y2,x1,x2) are uploaded once and stay resident in HBM. */
+ * (n,H,W,3) u8 BGR and coords (n,4) int32 = (y1,y2,x1,x2) are uploaded once and stay resident in HBM.
+ * frames == NULL creates a FRAME-FREE avatar: only faces and coords go to the device (H, W still validate the coords), the
+ * caller keeps the frames, and only the *_region entry points composite for it.  The full-frame forms (ltb_w2l_paste,
+ * ltb_w2l_paste_pred, ltb_w2l_paste_batch, ltb_w2l_infer_paste, ltb_w2l_infer_slots, ltb_w2l_step_async,
+ * ltb_w2l_step_e2e_async) fail with a message for it and leave the session usable. */
 int ltb_w2l_avatar_create(const uint8_t* faces, const uint8_t* frames, const int32_t* coords, int n, int H, int W,
                           ltb_w2l_avatar** out);
 int ltb_w2l_avatar_destroy(ltb_w2l_avatar* a);
+/* the avatar's largest paste rectangle (max y2-y1, max x2-x1 over its frames): the per-slot pitch of region outputs */
+int ltb_w2l_avatar_region_max(const ltb_w2l_avatar* a, int* rh_max, int* rw_max);
+/* cudaMemGetInfo of the current device (the plugins decide an avatar's residency from it) */
+int ltb_mem_get_info(size_t* free_bytes, size_t* total_bytes);
 
 /* ---- session (one avatar stream) -------------------------------------------------------------------- */
 #define LTB_SESSION_KEEP_LAYERS 1 /* keep every layer's activations (debug / per-layer parity tests) */
@@ -109,6 +117,18 @@ typedef struct ltb_w2l_slot {
   const float* mel;   /* host float32 [80,16] */
 } ltb_w2l_slot;
 int ltb_w2l_infer_slots(ltb_w2l_session* s, const ltb_w2l_slot* slots, int nslots, uint8_t* out_frames);
+
+/* Region forms of the composite, for frame-free avatars (and usable with any avatar): the device writes only the paste
+ * rectangle, cv2.resize(pred.astype(u8), (x2-x1, y2-y1)) of avatars/wav2lip_avatar.py:141-147, and the host writes it into its
+ * own copy of frame idx at (y1, x1).  Packed outputs are uint8 [count][rh_max][rw_max][3] with (rh_max, rw_max) of the SESSION's
+ * avatar (ltb_w2l_avatar_region_max); slot i's rectangle of its coords (h, w) is out[i][0:h][0:w], the rest is unspecified.
+ *   infer_paste_region: ltb_w2l_infer_paste with region output (count = batch).  Synchronous.
+ *   infer_slots_region: ltb_w2l_infer_slots with region output (count = nslots).  Slot avatars may have any frame size; each
+ *                       rectangle must fit (rh_max, rw_max) of the session's avatar.  Synchronous.
+ *   paste_pred_region:  ltb_w2l_paste_pred with region output, tightly packed uint8 [y2-y1][x2-x1][3].  Synchronous. */
+int ltb_w2l_infer_paste_region(ltb_w2l_session* s, int index, const float* mel, uint8_t* out_regions);
+int ltb_w2l_infer_slots_region(ltb_w2l_session* s, const ltb_w2l_slot* slots, int nslots, uint8_t* out_regions);
+int ltb_w2l_paste_pred_region(ltb_w2l_session* s, const float* pred, int idx, uint8_t* out_region);
 
 /* mel windows from the PCM buffer already resident on the device (uploaded by ltb_w2l_set_pcm):
  * the device-resident form of MelASR.run_step's feature extraction.  Asynchronous. */
@@ -248,6 +268,10 @@ int ltb_op_head_sigmoid255(ltb_ctx* c, const void* x, const float* w3x32, const 
  * explicit_idx (>= 0) or mirror_index(nf, index + j).  Bit-exact with OpenCV. */
 int ltb_op_ul_paste(ltb_ctx* c, const void* frames, const void* faces, const void* coords, const float* pred, void* out, int nf, int H, int W,
                     int index, int explicit_idx, int slot0, int count);
+/* region twin for frame-free avatars: only the bbox rectangle cv2.resize(crop, (x2-x1, y2-y1)), no frame read.  Job j writes
+ * out[j][0:y2-y1][0:x2-x1] of a packed uint8 [count][rh][rw][3] buffer (rh, rw >= every box of the jobs); the host pastes it. */
+int ltb_op_ul_paste_region(ltb_ctx* c, const void* faces, const void* coords, const float* pred, void* out, int nf, int rh, int rw, int index,
+                           int explicit_idx, int slot0, int count);
 /* Audio2Feature.get_hubert_from_16k_speech front end, avatars/ultralight/audio2feature.py:14-20: Wav2Vec2 processor normalisation
  * (stats[2] = mean, 1/sqrt(var + 1e-7)) fused with HubertModel's conv layer 0 (w fp32 [C][10], stride 5) -> fp16 [(n-10)/5+1][C] */
 int ltb_op_hubert_conv0(ltb_ctx* c, const float* pcm, int n, const float* w, const float* bias, int C, float* stats, void* out);
@@ -285,6 +309,12 @@ typedef struct ltb_mt_paste_op {
   const void* frames; const void* coords; const void* crop; const void* masks; const void* mask_off; const void* pred; void* out;
   int nf, H, W, index, explicit_idx, slot0, count;
   int pred_hw;   /* side of the square prediction: 256 (the reference, vae.py:15) or 512 (64x64 latents); 0 = 256 */
+  /* region form (frame-free avatars; zero = the full-frame form above): body = the crop box of every original frame, packed exactly
+   * like the masks (same shapes, same mask_off); frames is not read and may be NULL.  Job j writes only its blended crop box,
+   * out[j][0:y_e-y_s][0:x_e-x_s] of a packed uint8 [count][region_h][region_w][3] buffer (region_h/w >= every crop box of the jobs);
+   * nothing outside the crop box changes, so the host pastes it into its own copy of the frame. */
+  const void* body;
+  int region_h, region_w;
 } ltb_mt_paste_op;
 int ltb_op_mt_paste(ltb_ctx* c, const ltb_mt_paste_op* d);
 

@@ -31,7 +31,8 @@ class ConvOp(C.Structure):
 
 class MtPasteOp(C.Structure):
     _fields_ = ([(n, C.c_void_p) for n in ("frames", "coords", "crop", "masks", "mask_off", "pred", "out")] +
-                [(n, C.c_int) for n in ("nf", "H", "W", "index", "explicit_idx", "slot0", "count", "pred_hw")])
+                [(n, C.c_int) for n in ("nf", "H", "W", "index", "explicit_idx", "slot0", "count", "pred_hw")] +
+                [("body", C.c_void_p), ("region_h", C.c_int), ("region_w", C.c_int)])
 
 
 class W2LSlot(C.Structure):
@@ -55,6 +56,8 @@ _SIGS = {
     "ltb_w2l_avatar_create": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                         C.POINTER(C.c_void_p)]),
     "ltb_w2l_avatar_destroy": (C.c_int, [C.c_void_p]),
+    "ltb_w2l_avatar_region_max": (C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "ltb_mem_get_info": (C.c_int, [C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)]),
     "ltb_w2l_session_create": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                          C.POINTER(C.c_void_p)]),
     "ltb_w2l_session_destroy": (C.c_int, [C.c_void_p]),
@@ -66,6 +69,9 @@ _SIGS = {
     "ltb_w2l_paste_batch": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
     "ltb_w2l_infer_paste": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "ltb_w2l_infer_slots": (C.c_int, [C.c_void_p, C.POINTER(W2LSlot), C.c_int, C.c_void_p]),
+    "ltb_w2l_infer_paste_region": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "ltb_w2l_infer_slots_region": (C.c_int, [C.c_void_p, C.POINTER(W2LSlot), C.c_int, C.c_void_p]),
+    "ltb_w2l_paste_pred_region": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "ltb_w2l_mel_resident": (C.c_int, [C.c_void_p]),
     "ltb_w2l_step_async": (C.c_int, [C.c_void_p, C.c_int]),
     "ltb_w2l_forward_async": (C.c_int, [C.c_void_p, C.c_int]),
@@ -118,6 +124,8 @@ _SIGS = {
     "ltb_op_head_sigmoid255": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_void_p]),
     "ltb_op_ul_paste": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
                                   C.c_int, C.c_int, C.c_int]),
+    "ltb_op_ul_paste_region": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int,
+                                         C.c_int, C.c_int, C.c_int]),
     "ltb_op_hubert_conv0": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "ltb_op_hubert_pos_conv": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ltb_op_hubert_slice": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int,

@@ -83,7 +83,7 @@ inline cudaError_t launch_kernel_plain(void (*kernel)(KArgs...), dim3 grid, dim3
 // paste launch serves frames of different sessions (different avatars, unrelated frame indices)
 struct SlotDesc {
   const uint8_t* face;    // u8 [256,256,3] BGR crop of this slot
-  const uint8_t* frame;   // u8 [H,W,3] full frame the prediction is pasted into
+  const uint8_t* frame;   // u8 [H,W,3] full frame the prediction is pasted into (nullptr: frame-free avatar, region paste)
   int y1, y2, x1, x2;     // paste rectangle (wav2lip coords.pkl order)
 };
 
@@ -113,5 +113,9 @@ size_t mel_scratch_mel_doubles(int nsamp);
 //   frame index of job i = explicit_idx (>= 0, count must be 1) or mirror_index(nf, index + i); prediction slot = slot0 + i
 cudaError_t launch_w2l_paste(const uint8_t* frames, const int* coords, int nf, int H, int W, const float* pred, int slot0,
                              int index, int explicit_idx, int count, uint8_t* out, cudaStream_t st, const SlotDesc* slots = nullptr);
+// same jobs, region form: job i writes only its paste rectangle (h, w) into out[i][0:h][0:w] of a packed u8 [count][rh][rw][3]
+// buffer (rh >= h, rw >= w); no frame is read
+cudaError_t launch_w2l_paste_region(const int* coords, int nf, const float* pred, int slot0, int index, int explicit_idx, int count,
+                                    uint8_t* out, int rh, int rw, cudaStream_t st, const SlotDesc* slots = nullptr);
 
 }  // namespace ltb

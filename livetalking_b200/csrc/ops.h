@@ -34,6 +34,9 @@ cudaError_t launch_upsample_bilinear2x(const __half* x, int N, int H, int W, int
 cudaError_t launch_ul_prep(const uint8_t* faces, int nf, const int* d_index, int B, __half* out, cudaStream_t st);
 cudaError_t launch_ul_paste(const uint8_t* frames, const uint8_t* faces, const int* coords, const float* pred, uint8_t* out, int nf, int H, int W,
                             int index, int explicit_idx, int slot0, int count, cudaStream_t st);
+// region form: job j's bbox rectangle into out[j][0:h][0:w] of a packed u8 [count][rh][rw][3] buffer, no frame read
+cudaError_t launch_ul_paste_region(const uint8_t* faces, const int* coords, const float* pred, uint8_t* out, int nf, int rh, int rw, int index,
+                                   int explicit_idx, int slot0, int count, cudaStream_t st);
 cudaError_t launch_hubert_conv0(const float* pcm, int n, const float* w, const float* bias, int C, float* stats, __half* out, cudaStream_t st);
 cudaError_t launch_hubert_pos_conv(const __half* h, int T, int D, int groups, int K, const __half* w, const float* bias, __half* out,
                                    cudaStream_t st);
@@ -64,6 +67,8 @@ struct MtPasteArgs {
   int nf, H, W;
   int index, explicit_idx, slot0;
   int S;                     // prediction side: 256 (reference), 512 for the 64x64-latent configuration
+  const uint8_t* body;       // != nullptr: region form (frame-free avatar): body crops packed like the masks; out is [count][rh][rw][3]
+  int rh, rw;
 };
 cudaError_t launch_mt_paste(const MtPasteArgs& a, int count, cudaStream_t st);
 

@@ -442,6 +442,17 @@ int ltb_op_ul_paste(ltb_ctx* c, const void* frames, const void* faces, const voi
   c->launches += 1;
   return 0;
 }
+int ltb_op_ul_paste_region(ltb_ctx* c, const void* faces, const void* coords, const float* pred, void* out, int nf, int rh, int rw, int index,
+                           int explicit_idx, int slot0, int count) {
+  if (!c || !faces || !coords || !pred || !out || nf < 1 || count < 1 || rh < 1 || rw < 1) return LTB_FAIL("ul_paste_region: bad argument");
+  if (explicit_idx >= nf) return LTB_FAIL("ul_paste_region: frame index out of range");
+  LTB_CTX_ENTER(c);
+  cudaError_t e = launch_ul_paste_region(static_cast<const uint8_t*>(faces), static_cast<const int*>(coords), pred, static_cast<uint8_t*>(out), nf,
+                                         rh, rw, index, explicit_idx, slot0, count, c->st);
+  if (e != cudaSuccess) return LTB_FAIL(std::string("ul_paste_region: ") + cudaGetErrorString(e));
+  c->launches += 1;
+  return 0;
+}
 int ltb_op_hubert_conv0(ltb_ctx* c, const float* pcm, int n, const float* w, const float* bias, int C, float* stats, void* out) {
   if (!c || !pcm || !w || !stats || !out) return LTB_FAIL("hubert_conv0: null argument");
   LTB_CTX_ENTER(c);
@@ -550,6 +561,11 @@ int ltb_op_mt_paste(ltb_ctx* c, const ltb_mt_paste_op* d) {
   a.explicit_idx = d->explicit_idx;
   a.slot0 = d->slot0;
   a.S = d->pred_hw > 0 ? d->pred_hw : 256;
+  a.body = static_cast<const uint8_t*>(d->body);
+  a.rh = d->region_h;
+  a.rw = d->region_w;
+  if (!a.body && !a.frames) return LTB_FAIL("mt_paste: frames == NULL (frame-free avatar): set body to its body crops for the region form");
+  if (a.body && (a.rh < 1 || a.rw < 1)) return LTB_FAIL("mt_paste: the region form needs region_h, region_w >= the crop boxes");
   cudaError_t e = launch_mt_paste(a, d->count, c->st);
   if (e != cudaSuccess) return LTB_FAIL(std::string("mt_paste: ") + cudaGetErrorString(e));
   c->launches += 1;

@@ -10,6 +10,55 @@
 
 namespace ltb {
 
+// One pixel of cv2.resize(pred.astype(u8), (dw, dh)) at (dy, dx) of the paste rectangle: the per-pixel arithmetic shared by the
+// full-frame kernels and the region kernel.  The row taps depend on dy only and are set up once per row.
+struct W2LRowTaps {
+  bool same, area;
+  int dy, sy0, sy1, b0, b1;
+  double scale_x;
+};
+
+__device__ __forceinline__ W2LRowTaps w2l_row_taps(int dy, int dw, int dh) {
+  W2LRowTaps t;
+  t.same = (dw == 256 && dh == 256);
+  t.area = (dw == 128 && dh == 128);
+  t.dy = dy;
+  int sy = 0;
+  t.b0 = 2048;
+  t.b1 = 0;
+  if (!t.same && !t.area) cv_tap(dy, 1.0 / ((double)dh / 256.0), 256, false, sy, t.b0, t.b1);
+  t.sy0 = min(max(sy, 0), 255);
+  t.sy1 = min(max(sy + 1, 0), 255);
+  t.scale_x = 1.0 / ((double)dw / 256.0);
+  return t;
+}
+
+__device__ __forceinline__ void w2l_resize_px(const float* pred, const W2LRowTaps& t, int dx, int v3[3]) {
+  if (t.same) {
+    const float* p = pred + ((size_t)t.dy * 256 + dx) * 3;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) v3[c] = trunc_u8(p[c]);
+  } else if (t.area) {
+    const float* p = pred + ((size_t)(2 * t.dy) * 256 + 2 * dx) * 3;
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+      v3[c] = (trunc_u8(p[c]) + trunc_u8(p[3 + c]) + trunc_u8(p[768 + c]) + trunc_u8(p[771 + c]) + 2) >> 2;
+  } else {
+    int sx, a0, a1;
+    cv_tap(dx, t.scale_x, 256, true, sx, a0, a1);
+    const int sx1 = min(sx + 1, 255);
+    const float* r0 = pred + (size_t)t.sy0 * 768;
+    const float* r1 = pred + (size_t)t.sy1 * 768;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      const int S0 = trunc_u8(r0[sx * 3 + c]) * a0 + trunc_u8(r0[sx1 * 3 + c]) * a1;
+      const int S1 = trunc_u8(r1[sx * 3 + c]) * a0 + trunc_u8(r1[sx1 * 3 + c]) * a1;
+      const int v = (((t.b0 * (S0 >> 4)) >> 16) + ((t.b1 * (S1 >> 4)) >> 16) + 2) >> 2;
+      v3[c] = min(max(v, 0), 255);
+    }
+  }
+}
+
 struct PasteArgs {
   const uint8_t* frames;  // [nf,H,W,3]
   const int* coords;      // [nf,4] = (y1,y2,x1,x2)
@@ -40,44 +89,18 @@ __global__ void __launch_bounds__(256) w2l_paste_kernel(const PasteArgs a) {
   }
   uint8_t* orow = a.out + ((size_t)job * a.H + y) * a.W * 3;
   const float* pred = a.pred + (size_t)(a.slot0 + job) * 256 * 256 * 3;
-  const int dw = x2 - x1, dh = y2 - y1;
   const int npx = min(4, a.W - xg);
   uint8_t px[12];
 #pragma unroll
   for (int i = 0; i < 12; ++i) px[i] = (i < npx * 3) ? frow[xg * 3 + i] : 0;
   if (y >= y1 && y < y2 && xg + npx > x1 && xg < x2) {
-    const int dy = y - y1;
-    const bool same = (dw == 256 && dh == 256);
-    const bool area = (dw == 128 && dh == 128);
-    int sy = 0, b0 = 2048, b1 = 0;
-    if (!same && !area) cv_tap(dy, 1.0 / ((double)dh / 256.0), 256, false, sy, b0, b1);
-    const int sy0 = min(max(sy, 0), 255), sy1 = min(max(sy + 1, 0), 255);
+    const W2LRowTaps t = w2l_row_taps(y - y1, x2 - x1, y2 - y1);
     for (int i = 0; i < npx; ++i) {
       const int x = xg + i;
       if (x < x1 || x >= x2) continue;
-      const int dx = x - x1;
-      if (same) {
-        const float* p = pred + ((size_t)dy * 256 + dx) * 3;
-        for (int c = 0; c < 3; ++c) px[i * 3 + c] = (uint8_t)trunc_u8(p[c]);
-      } else if (area) {
-        const float* p = pred + ((size_t)(2 * dy) * 256 + 2 * dx) * 3;
-        for (int c = 0; c < 3; ++c) {
-          const int s = trunc_u8(p[c]) + trunc_u8(p[3 + c]) + trunc_u8(p[768 + c]) + trunc_u8(p[771 + c]);
-          px[i * 3 + c] = (uint8_t)((s + 2) >> 2);
-        }
-      } else {
-        int sx, a0, a1;
-        cv_tap(dx, 1.0 / ((double)dw / 256.0), 256, true, sx, a0, a1);
-        const int sx1 = min(sx + 1, 255);
-        const float* r0 = pred + (size_t)sy0 * 768;
-        const float* r1 = pred + (size_t)sy1 * 768;
-        for (int c = 0; c < 3; ++c) {
-          const int S0 = trunc_u8(r0[sx * 3 + c]) * a0 + trunc_u8(r0[sx1 * 3 + c]) * a1;
-          const int S1 = trunc_u8(r1[sx * 3 + c]) * a0 + trunc_u8(r1[sx1 * 3 + c]) * a1;
-          const int v = (((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2;
-          px[i * 3 + c] = (uint8_t)min(max(v, 0), 255);
-        }
-      }
+      int v3[3];
+      w2l_resize_px(pred, t, x - x1, v3);
+      for (int c = 0; c < 3; ++c) px[i * 3 + c] = (uint8_t)v3[c];
     }
   }
   if (npx == 4 && ((a.W * 3) % 4 == 0)) {
@@ -122,43 +145,13 @@ __global__ void __launch_bounds__(256) w2l_paste_vec_kernel(const PasteArgs a, i
     }
     if (y >= y1 && y < y2 && xg + 16 > x1 && xg < x2) {
       const float* pred = a.pred + (size_t)(a.slot0 + job) * 256 * 256 * 3;
-      const int dw = x2 - x1, dh = y2 - y1;
-      const int dy = y - y1;
-      const bool same = (dw == 256 && dh == 256);
-      const bool area = (dw == 128 && dh == 128);
-      int sy = 0, b0 = 2048, b1 = 0;
-      if (!same && !area) cv_tap(dy, 1.0 / ((double)dh / 256.0), 256, false, sy, b0, b1);
-      const int sy0 = min(max(sy, 0), 255), sy1 = min(max(sy + 1, 0), 255);
-      const double scale_x = 1.0 / ((double)dw / 256.0);
+      const W2LRowTaps t = w2l_row_taps(y - y1, x2 - x1, y2 - y1);
 #pragma unroll
       for (int i = 0; i < 16; ++i) {
         const int x = xg + i;
         if (x < x1 || x >= x2) continue;
-        const int dx = x - x1;
         int v3[3];
-        if (same) {
-          const float* p = pred + ((size_t)dy * 256 + dx) * 3;
-#pragma unroll
-          for (int c = 0; c < 3; ++c) v3[c] = trunc_u8(p[c]);
-        } else if (area) {
-          const float* p = pred + ((size_t)(2 * dy) * 256 + 2 * dx) * 3;
-#pragma unroll
-          for (int c = 0; c < 3; ++c)
-            v3[c] = (trunc_u8(p[c]) + trunc_u8(p[3 + c]) + trunc_u8(p[768 + c]) + trunc_u8(p[771 + c]) + 2) >> 2;
-        } else {
-          int sx, a0, a1;
-          cv_tap(dx, scale_x, 256, true, sx, a0, a1);
-          const int sx1 = min(sx + 1, 255);
-          const float* r0 = pred + (size_t)sy0 * 768;
-          const float* r1 = pred + (size_t)sy1 * 768;
-#pragma unroll
-          for (int c = 0; c < 3; ++c) {
-            const int S0 = trunc_u8(r0[sx * 3 + c]) * a0 + trunc_u8(r0[sx1 * 3 + c]) * a1;
-            const int S1 = trunc_u8(r1[sx * 3 + c]) * a0 + trunc_u8(r1[sx1 * 3 + c]) * a1;
-            const int v = (((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2;
-            v3[c] = min(max(v, 0), 255);
-          }
-        }
+        w2l_resize_px(pred, t, x - x1, v3);
 #pragma unroll
         for (int c = 0; c < 3; ++c) {
           const int bi = i * 3 + c;   // static after unrolling: byte bi of the 48-byte group
@@ -198,6 +191,46 @@ cudaError_t launch_w2l_paste(const uint8_t* frames, const int* coords, int nf, i
   }
   dim3 grid((W + 1023) / 1024, H, count);
   w2l_paste_kernel<<<grid, 256, 0, st>>>(a);
+  return cudaGetLastError();
+}
+
+// Region form for frame-free avatars: only the paste rectangle of job j, written to out[j][0:dh][0:dw] of a packed
+// [count][rh][rw][3] buffer.  No frame is read; the host writes the rectangle into its own copy of the frame.  One thread = one pixel.
+__global__ void __launch_bounds__(256) w2l_paste_region_kernel(const PasteArgs a, int rh, int rw) {
+  const int job = blockIdx.z;
+  const int dy = blockIdx.y;
+  const int dx = blockIdx.x * 256 + threadIdx.x;
+  int y1, y2, x1, x2;
+  if (a.slots) {
+    const SlotDesc sd = a.slots[job];
+    y1 = sd.y1, y2 = sd.y2, x1 = sd.x1, x2 = sd.x2;
+  } else {
+    const int idx = a.explicit_idx >= 0 ? a.explicit_idx : mirror_index_p(a.nf, a.index + job);
+    y1 = a.coords[idx * 4 + 0], y2 = a.coords[idx * 4 + 1], x1 = a.coords[idx * 4 + 2], x2 = a.coords[idx * 4 + 3];
+  }
+  const int dw = x2 - x1, dh = y2 - y1;
+  if (dy >= dh || dx >= dw) return;
+  const float* pred = a.pred + (size_t)(a.slot0 + job) * 256 * 256 * 3;
+  int v3[3];
+  w2l_resize_px(pred, w2l_row_taps(dy, dw, dh), dx, v3);
+  uint8_t* o = a.out + (((size_t)job * rh + dy) * rw + dx) * 3;
+#pragma unroll
+  for (int c = 0; c < 3; ++c) o[c] = (uint8_t)v3[c];
+}
+
+cudaError_t launch_w2l_paste_region(const int* coords, int nf, const float* pred, int slot0, int index, int explicit_idx, int count,
+                                    uint8_t* out, int rh, int rw, cudaStream_t st, const SlotDesc* slots) {
+  PasteArgs a{};
+  a.slots = slots;
+  a.coords = coords;
+  a.pred = pred;
+  a.out = out;
+  a.nf = nf;
+  a.index = index;
+  a.explicit_idx = explicit_idx;
+  a.slot0 = slot0;
+  dim3 grid((rw + 255) / 256, rh, count);
+  w2l_paste_region_kernel<<<grid, 256, 0, st>>>(a, rh, rw);
   return cudaGetLastError();
 }
 

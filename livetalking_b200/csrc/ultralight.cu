@@ -161,6 +161,33 @@ __device__ __forceinline__ int ul_src(const uint8_t* __restrict__ face, const fl
   return face[(sy * 168 + sx) * 3 + c];
 }
 
+// pixel (dy, dx) of cv2.resize(crop_img_ori, (dw, dh)): the per-pixel arithmetic shared by the full-frame and the region kernels
+__device__ __forceinline__ void ul_resize_px(const uint8_t* __restrict__ face, const float* __restrict__ pred, int dy, int dx, int dw, int dh,
+                                             uint8_t px[3]) {
+  constexpr int S = 168;
+  if (dw == S && dh == S) {
+#pragma unroll
+    for (int c = 0; c < 3; ++c) px[c] = (uint8_t)ul_src(face, pred, dy, dx, c);
+  } else if (2 * dw == S && 2 * dh == S) {   // exact 2x shrink: OpenCV's INTER_LINEAR takes the 2x2 area path
+#pragma unroll
+    for (int c = 0; c < 3; ++c)
+      px[c] = (uint8_t)((ul_src(face, pred, 2 * dy, 2 * dx, c) + ul_src(face, pred, 2 * dy, 2 * dx + 1, c) + ul_src(face, pred, 2 * dy + 1, 2 * dx, c) +
+                         ul_src(face, pred, 2 * dy + 1, 2 * dx + 1, c) + 2) >> 2);
+  } else {
+    int sy, b0, b1, sx, a0, a1;
+    cv_tap(dy, 1.0 / ((double)dh / (double)S), S, false, sy, b0, b1);
+    cv_tap(dx, 1.0 / ((double)dw / (double)S), S, true, sx, a0, a1);
+    const int sy0 = min(max(sy, 0), S - 1), sy1 = min(max(sy + 1, 0), S - 1), sx1 = min(sx + 1, S - 1);
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+      const int S0 = ul_src(face, pred, sy0, sx, c) * a0 + ul_src(face, pred, sy0, sx1, c) * a1;
+      const int S1 = ul_src(face, pred, sy1, sx, c) * a0 + ul_src(face, pred, sy1, sx1, c) * a1;
+      const int v = (((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2;
+      px[c] = (uint8_t)min(max(v, 0), 255);
+    }
+  }
+}
+
 __global__ void __launch_bounds__(256) ul_paste_kernel(const UlPasteArgs a) {
   pdl_launch_dependents();   // a PDL-launched successor (the conv kernels) may start its prologue now; it waits before reading
   const int job = blockIdx.z, y = blockIdx.y;
@@ -171,33 +198,8 @@ __global__ void __launch_bounds__(256) ul_paste_kernel(const UlPasteArgs a) {
   const uint8_t* body = a.frames + (((size_t)idx * a.H + y) * a.W + x) * 3;
   uint8_t* o = a.out + (((size_t)job * a.H + y) * a.W + x) * 3;
   uint8_t px[3] = {body[0], body[1], body[2]};
-  if (y >= y1 && y < y2 && x >= x1 && x < x2) {
-    constexpr int S = 168;
-    const uint8_t* face = a.faces + (size_t)idx * S * S * 3;
-    const float* pred = a.pred + (size_t)(a.slot0 + job) * 160 * 160 * 3;
-    const int dw = x2 - x1, dh = y2 - y1, dy = y - y1, dx = x - x1;
-    if (dw == S && dh == S) {
-#pragma unroll
-      for (int c = 0; c < 3; ++c) px[c] = (uint8_t)ul_src(face, pred, dy, dx, c);
-    } else if (2 * dw == S && 2 * dh == S) {   // exact 2x shrink: OpenCV's INTER_LINEAR takes the 2x2 area path
-#pragma unroll
-      for (int c = 0; c < 3; ++c)
-        px[c] = (uint8_t)((ul_src(face, pred, 2 * dy, 2 * dx, c) + ul_src(face, pred, 2 * dy, 2 * dx + 1, c) + ul_src(face, pred, 2 * dy + 1, 2 * dx, c) +
-                           ul_src(face, pred, 2 * dy + 1, 2 * dx + 1, c) + 2) >> 2);
-    } else {
-      int sy, b0, b1, sx, a0, a1;
-      cv_tap(dy, 1.0 / ((double)dh / (double)S), S, false, sy, b0, b1);
-      cv_tap(dx, 1.0 / ((double)dw / (double)S), S, true, sx, a0, a1);
-      const int sy0 = min(max(sy, 0), S - 1), sy1 = min(max(sy + 1, 0), S - 1), sx1 = min(sx + 1, S - 1);
-#pragma unroll
-      for (int c = 0; c < 3; ++c) {
-        const int S0 = ul_src(face, pred, sy0, sx, c) * a0 + ul_src(face, pred, sy0, sx1, c) * a1;
-        const int S1 = ul_src(face, pred, sy1, sx, c) * a0 + ul_src(face, pred, sy1, sx1, c) * a1;
-        const int v = (((b0 * (S0 >> 4)) >> 16) + ((b1 * (S1 >> 4)) >> 16) + 2) >> 2;
-        px[c] = (uint8_t)min(max(v, 0), 255);
-      }
-    }
-  }
+  if (y >= y1 && y < y2 && x >= x1 && x < x2)
+    ul_resize_px(a.faces + (size_t)idx * 168 * 168 * 3, a.pred + (size_t)(a.slot0 + job) * 160 * 160 * 3, y - y1, x - x1, x2 - x1, y2 - y1, px);
   o[0] = px[0];
   o[1] = px[1];
   o[2] = px[2];
@@ -208,6 +210,30 @@ cudaError_t launch_ul_paste(const uint8_t* frames, const uint8_t* faces, const i
   UlPasteArgs a{frames, faces, coords, pred, out, nf, H, W, index, explicit_idx, slot0};
   dim3 grid((W + 255) / 256, H, count);
   return launch_kernel_plain(ul_paste_kernel, dim3(grid), dim3(256), 0, st, a);
+}
+
+// Region form for frame-free avatars: job j writes only its bbox rectangle, out[j][0:dh][0:dw] of a packed [count][rh][rw][3] buffer;
+// no frame is read (a.frames, a.H, a.W unused).
+__global__ void __launch_bounds__(256) ul_paste_region_kernel(const UlPasteArgs a, int rh, int rw) {
+  pdl_launch_dependents();
+  const int job = blockIdx.z, dy = blockIdx.y;
+  const int dx = blockIdx.x * 256 + threadIdx.x;
+  const int idx = a.explicit_idx >= 0 ? a.explicit_idx : mirror_index_p(a.nf, a.index + job);
+  const int x1 = a.coords[idx * 4 + 0], y1 = a.coords[idx * 4 + 1], x2 = a.coords[idx * 4 + 2], y2 = a.coords[idx * 4 + 3];
+  if (dy >= y2 - y1 || dx >= x2 - x1) return;
+  uint8_t px[3];
+  ul_resize_px(a.faces + (size_t)idx * 168 * 168 * 3, a.pred + (size_t)(a.slot0 + job) * 160 * 160 * 3, dy, dx, x2 - x1, y2 - y1, px);
+  uint8_t* o = a.out + (((size_t)job * rh + dy) * rw + dx) * 3;
+  o[0] = px[0];
+  o[1] = px[1];
+  o[2] = px[2];
+}
+
+cudaError_t launch_ul_paste_region(const uint8_t* faces, const int* coords, const float* pred, uint8_t* out, int nf, int rh, int rw, int index,
+                                   int explicit_idx, int slot0, int count, cudaStream_t st) {
+  UlPasteArgs a{nullptr, faces, coords, pred, out, nf, 0, 0, index, explicit_idx, slot0};
+  dim3 grid((rw + 255) / 256, rh, count);
+  return launch_kernel_plain(ul_paste_region_kernel, dim3(grid), dim3(256), 0, st, a, rh, rw);
 }
 
 }  // namespace ltb

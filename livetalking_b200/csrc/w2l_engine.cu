@@ -9,6 +9,7 @@
 //   pred      [B,256,256,3]   f32            : sigmoid*255, the reference's inference_batch return layout
 //   frames_out[B,H,W,3]       u8             : composited frames
 // Reference topology: avatars/wav2lip/models/wav2lip_v2.py:12-91, forward :123-163.
+#include <algorithm>
 #include <cstring>
 #include <memory>
 #include <mutex>
@@ -199,9 +200,10 @@ struct ltb_w2l_avatar {
   int device = 0;
   int n = 0, H = 0, W = 0;
   uint8_t* faces = nullptr;
-  uint8_t* frames = nullptr;
+  uint8_t* frames = nullptr;   // nullptr: frame-free avatar (the host keeps the frames; only region outputs are produced)
   int* coords = nullptr;
   std::vector<int> coords_host;
+  int rh_max = 0, rw_max = 0;  // largest paste rectangle: the per-slot pitch of region outputs
 };
 
 namespace ltb {
@@ -803,29 +805,47 @@ int ltb_w2l_avatar_destroy(ltb_w2l_avatar* a);
 
 int ltb_w2l_avatar_create(const uint8_t* faces, const uint8_t* frames, const int32_t* coords, int n, int H, int W,
                           ltb_w2l_avatar** out) {
-  if (!faces || !frames || !coords || !out || n <= 0 || H <= 0 || W <= 0) return LTB_FAIL("bad avatar arguments");
+  if (!faces || !coords || !out || n <= 0 || H <= 0 || W <= 0) return LTB_FAIL("bad avatar arguments");
+  int rh_max = 0, rw_max = 0;
   for (int i = 0; i < n; ++i) {
     const int y1 = coords[i * 4], y2 = coords[i * 4 + 1], x1 = coords[i * 4 + 2], x2 = coords[i * 4 + 3];
     if (y1 < 0 || x1 < 0 || y2 > H || x2 > W || y2 <= y1 || x2 <= x1)
       return LTB_FAIL("avatar coords[" + std::to_string(i) + "] outside the frame");
+    rh_max = std::max(rh_max, y2 - y1);
+    rw_max = std::max(rw_max, x2 - x1);
   }
   auto* a = new ltb_w2l_avatar();
   a->n = n;
   a->H = H;
   a->W = W;
+  a->rh_max = rh_max;
+  a->rw_max = rw_max;
   a->coords_host.assign(coords, coords + (size_t)n * 4);
   cudaError_t e = cudaGetDevice(&a->device);
   if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&a->faces), (size_t)n * 65536 * 3);
-  if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&a->frames), (size_t)n * H * W * 3);
+  if (e == cudaSuccess && frames) e = cudaMalloc(reinterpret_cast<void**>(&a->frames), (size_t)n * H * W * 3);
   if (e == cudaSuccess) e = cudaMalloc(reinterpret_cast<void**>(&a->coords), (size_t)n * 4 * sizeof(int));
   if (e == cudaSuccess) e = cudaMemcpy(a->faces, faces, (size_t)n * 65536 * 3, cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaMemcpy(a->frames, frames, (size_t)n * H * W * 3, cudaMemcpyHostToDevice);
+  if (e == cudaSuccess && frames) e = cudaMemcpy(a->frames, frames, (size_t)n * H * W * 3, cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaMemcpy(a->coords, coords, (size_t)n * 4 * sizeof(int), cudaMemcpyHostToDevice);
   if (e != cudaSuccess) {
     ltb_w2l_avatar_destroy(a);
     return LTB_FAIL(std::string("avatar upload: ") + cudaGetErrorString(e));
   }
   *out = a;
+  return 0;
+}
+
+int ltb_w2l_avatar_region_max(const ltb_w2l_avatar* a, int* rh_max, int* rw_max) {
+  if (!a || !rh_max || !rw_max) return LTB_FAIL("null argument");
+  *rh_max = a->rh_max;
+  *rw_max = a->rw_max;
+  return 0;
+}
+
+int ltb_mem_get_info(size_t* free_bytes, size_t* total_bytes) {
+  if (!free_bytes || !total_bytes) return LTB_FAIL("null argument");
+  LTB_CUDA(cudaMemGetInfo(free_bytes, total_bytes));
   return 0;
 }
 
@@ -932,7 +952,9 @@ int ltb_w2l_session_create(ltb_w2l_model* m, ltb_w2l_avatar* a, int batch, int s
   s->pred = static_cast<float*>(p);
   if (dev_alloc(s, (size_t)65536 * 3 * 4, &p, true)) return bail(1);
   s->pred_scratch = static_cast<float*>(p);
-  if (dev_alloc(s, (size_t)batch * a->H * a->W * 3, &p, true)) return bail(1);
+  // composite output: full frames, or (frame-free avatar) the packed paste rectangles [batch][rh_max][rw_max][3]
+  const size_t out_px = a->frames ? (size_t)a->H * a->W : (size_t)a->rh_max * a->rw_max;
+  if (dev_alloc(s, (size_t)batch * out_px * 3, &p, true)) return bail(1);
   s->frames_out = static_cast<uint8_t*>(p);
   if (dev_alloc(s, 256, &p, true)) return bail(1);
   s->d_index = static_cast<int*>(p);
@@ -1029,6 +1051,11 @@ int ltb_w2l_set_pcm(ltb_w2l_session* s, const float* pcm, int nsamples) {
   return 0;
 }
 
+static int need_frames(const ltb_w2l_avatar* a, const char* what) {
+  if (a->frames) return 0;
+  return LTB_FAIL(std::string(what) + ": the avatar was created frame-free (frames == NULL); use the *_region entry points");
+}
+
 static int forward_enqueue(ltb_w2l_session* s, int index, bool with_mel) {
   if (index < 0) return LTB_FAIL("negative index");
   if (s->ops.empty()) return LTB_FAIL("this session was created with LTB_SESSION_MEL_ONLY: it has no network");
@@ -1059,6 +1086,7 @@ int ltb_w2l_paste(ltb_w2l_session* s, int slot, int idx, uint8_t* out_frame) {
   if (s->ops.empty()) return LTB_FAIL("this session was created with LTB_SESSION_MEL_ONLY: it has no network");
   if (slot < 0 || slot >= s->B) return LTB_FAIL("paste: slot out of range");
   if (idx < 0 || idx >= s->a->n) return LTB_FAIL("paste: idx out of range");
+  if (need_frames(s->a, "ltb_w2l_paste")) return 1;
   if (enter(s)) return 1;
   std::lock_guard<std::mutex> lk(s->mu);
   const size_t fb = (size_t)s->a->H * s->a->W * 3;
@@ -1075,6 +1103,7 @@ int ltb_w2l_paste_pred(ltb_w2l_session* s, const float* pred, int idx, uint8_t* 
   if (!s || !pred || !out_frame) return LTB_FAIL("null argument");
   if (s->ops.empty()) return LTB_FAIL("this session was created with LTB_SESSION_MEL_ONLY: it has no network");
   if (idx < 0 || idx >= s->a->n) return LTB_FAIL("paste: idx out of range");
+  if (need_frames(s->a, "ltb_w2l_paste_pred")) return 1;
   if (enter(s)) return 1;
   std::lock_guard<std::mutex> lk(s->mu);
   const size_t fb = (size_t)s->a->H * s->a->W * 3;
@@ -1100,6 +1129,7 @@ int ltb_w2l_paste_batch(ltb_w2l_session* s, int index, uint8_t* out_frames) {
   if (!s) return LTB_FAIL("null session");
   if (s->ops.empty()) return LTB_FAIL("this session was created with LTB_SESSION_MEL_ONLY: it has no network");
   if (index < 0) return LTB_FAIL("negative index");
+  if (need_frames(s->a, "ltb_w2l_paste_batch")) return 1;
   if (enter(s)) return 1;
   std::lock_guard<std::mutex> lk(s->mu);
   if (paste_batch_enqueue(s, index)) return 1;
@@ -1113,6 +1143,7 @@ int ltb_w2l_paste_batch(ltb_w2l_session* s, int index, uint8_t* out_frames) {
 int ltb_w2l_infer_paste(ltb_w2l_session* s, int index, const float* mel, uint8_t* out_frames) {
   if (!s || !mel || !out_frames) return LTB_FAIL("null argument");
   if (s->ops.empty()) return LTB_FAIL("this session was created with LTB_SESSION_MEL_ONLY: it has no network");
+  if (need_frames(s->a, "ltb_w2l_infer_paste")) return 1;
   if (enter(s)) return 1;
   std::lock_guard<std::mutex> lk(s->mu);
   LTB_CUDA(cudaMemcpyAsync(s->mel, mel, (size_t)s->B * 1280 * 4, cudaMemcpyHostToDevice, s->st));
@@ -1123,36 +1154,94 @@ int ltb_w2l_infer_paste(ltb_w2l_session* s, int index, const float* mel, uint8_t
   return 0;
 }
 
-int ltb_w2l_infer_slots(ltb_w2l_session* s, const ltb_w2l_slot* slots, int nslots, uint8_t* out_frames) {
-  if (!s || !slots || !out_frames) return LTB_FAIL("null argument");
-  if (!s->d_slots) return LTB_FAIL("infer_slots: session was not created with LTB_SESSION_SLOTS");
-  if (nslots < 1 || nslots > s->B) return LTB_FAIL("infer_slots: 1 <= nslots <= batch");
+// Shared by both slot forms: validate the requests, stage the per-slot descriptors and mel windows, enqueue the forward.
+// region: slots may come from frame-free avatars of any frame size, but every rectangle must fit the session's region pitch.
+static int slots_forward_enqueue(ltb_w2l_session* s, const ltb_w2l_slot* slots, int nslots, bool region, const char* what) {
+  if (!s->d_slots) return LTB_FAIL(std::string(what) + ": session was not created with LTB_SESSION_SLOTS");
+  if (nslots < 1 || nslots > s->B) return LTB_FAIL(std::string(what) + ": 1 <= nslots <= batch");
   const int H = s->a->H, W = s->a->W;
   for (int i = 0; i < nslots; ++i) {
     const ltb_w2l_avatar* a = slots[i].avatar;
-    if (!a || !slots[i].mel) return LTB_FAIL("infer_slots: slot " + std::to_string(i) + " has a null avatar / mel");
-    if (a->device != s->device) return LTB_FAIL("infer_slots: avatar lives on another device");
-    if (a->H != H || a->W != W) return LTB_FAIL("infer_slots: all avatars of a batch must share the frame size of the session's avatar");
-    if (slots[i].idx < 0 || slots[i].idx >= a->n) return LTB_FAIL("infer_slots: frame index out of range");
+    const std::string slot = std::string(what) + ": slot " + std::to_string(i);
+    if (!a || !slots[i].mel) return LTB_FAIL(slot + " has a null avatar / mel");
+    if (a->device != s->device) return LTB_FAIL(slot + ": avatar lives on another device");
+    if (slots[i].idx < 0 || slots[i].idx >= a->n) return LTB_FAIL(slot + ": frame index out of range");
+    if (region) {
+      const int* c = &a->coords_host[(size_t)slots[i].idx * 4];
+      if (c[1] - c[0] > s->a->rh_max || c[3] - c[2] > s->a->rw_max)
+        return LTB_FAIL(slot + ": paste rectangle larger than the session avatar's largest (the region pitch)");
+    } else {
+      if (a->H != H || a->W != W) return LTB_FAIL(slot + ": all avatars of a batch must share the frame size of the session's avatar");
+      if (need_frames(a, what)) return 1;
+    }
   }
-  if (enter(s)) return 1;
-  std::lock_guard<std::mutex> lk(s->mu);
   for (int i = 0; i < s->B; ++i) {
     const ltb_w2l_slot& q = slots[i < nslots ? i : nslots - 1];   // unused slots repeat the last request (results discarded)
     const ltb_w2l_avatar* a = q.avatar;
     const int* c = &a->coords_host[(size_t)q.idx * 4];
-    s->h_slots[i] = SlotDesc{a->faces + (size_t)q.idx * 65536 * 3, a->frames + (size_t)q.idx * H * W * 3, c[0], c[1], c[2], c[3]};
+    const uint8_t* frame = a->frames ? a->frames + (size_t)q.idx * a->H * a->W * 3 : nullptr;
+    s->h_slots[i] = SlotDesc{a->faces + (size_t)q.idx * 65536 * 3, frame, c[0], c[1], c[2], c[3]};
     std::memcpy(s->h_mel_stage + (size_t)i * 1280, q.mel, 1280 * sizeof(float));
   }
   LTB_CUDA(cudaMemcpyAsync(s->d_slots, s->h_slots, (size_t)s->B * sizeof(SlotDesc), cudaMemcpyHostToDevice, s->st));
   LTB_CUDA(cudaMemcpyAsync(s->mel, s->h_mel_stage, (size_t)s->B * 1280 * 4, cudaMemcpyHostToDevice, s->st));
-  if (forward_enqueue(s, 0, false)) return 1;
+  return forward_enqueue(s, 0, false);
+}
+
+int ltb_w2l_infer_slots(ltb_w2l_session* s, const ltb_w2l_slot* slots, int nslots, uint8_t* out_frames) {
+  if (!s || !slots || !out_frames) return LTB_FAIL("null argument");
+  if (need_frames(s->a, "ltb_w2l_infer_slots")) return 1;
+  if (enter(s)) return 1;
+  std::lock_guard<std::mutex> lk(s->mu);
+  if (slots_forward_enqueue(s, slots, nslots, false, "infer_slots")) return 1;
+  const int H = s->a->H, W = s->a->W;
   cudaError_t e = launch_w2l_paste(nullptr, nullptr, 0, H, W, s->pred, 0, 0, -1, nslots, s->frames_out, s->st, s->d_slots);
   if (e != cudaSuccess) return LTB_FAIL(std::string("paste kernel: ") + cudaGetErrorString(e));
   s->launches += 1;
   LTB_CUDA(cudaMemcpyAsync(out_frames, s->frames_out, (size_t)nslots * H * W * 3, cudaMemcpyDeviceToHost, s->st));
   LTB_CUDA(cudaStreamSynchronize(s->st));
   return 0;
+}
+
+// ---- region forms (any avatar; the only composite forms for a frame-free one) ----
+static int region_enqueue_d2h(ltb_w2l_session* s, const float* pred, int index, int explicit_idx, int count, uint8_t* out,
+                              int rh, int rw, const SlotDesc* slots) {
+  cudaError_t e = launch_w2l_paste_region(s->a->coords, s->a->n, pred, 0, index, explicit_idx, count, s->frames_out, rh, rw, s->st,
+                                          slots);
+  if (e != cudaSuccess) return LTB_FAIL(std::string("region paste kernel: ") + cudaGetErrorString(e));
+  s->launches += 1;
+  LTB_CUDA(cudaMemcpyAsync(out, s->frames_out, (size_t)count * rh * rw * 3, cudaMemcpyDeviceToHost, s->st));
+  LTB_CUDA(cudaStreamSynchronize(s->st));
+  return 0;
+}
+
+int ltb_w2l_infer_paste_region(ltb_w2l_session* s, int index, const float* mel, uint8_t* out_regions) {
+  if (!s || !mel || !out_regions) return LTB_FAIL("null argument");
+  if (s->ops.empty()) return LTB_FAIL("this session was created with LTB_SESSION_MEL_ONLY: it has no network");
+  if (enter(s)) return 1;
+  std::lock_guard<std::mutex> lk(s->mu);
+  LTB_CUDA(cudaMemcpyAsync(s->mel, mel, (size_t)s->B * 1280 * 4, cudaMemcpyHostToDevice, s->st));
+  if (forward_enqueue(s, index, false)) return 1;
+  return region_enqueue_d2h(s, s->pred, index, -1, s->B, out_regions, s->a->rh_max, s->a->rw_max, nullptr);
+}
+
+int ltb_w2l_infer_slots_region(ltb_w2l_session* s, const ltb_w2l_slot* slots, int nslots, uint8_t* out_regions) {
+  if (!s || !slots || !out_regions) return LTB_FAIL("null argument");
+  if (enter(s)) return 1;
+  std::lock_guard<std::mutex> lk(s->mu);
+  if (slots_forward_enqueue(s, slots, nslots, true, "infer_slots_region")) return 1;
+  return region_enqueue_d2h(s, s->pred, 0, -1, nslots, out_regions, s->a->rh_max, s->a->rw_max, s->d_slots);
+}
+
+int ltb_w2l_paste_pred_region(ltb_w2l_session* s, const float* pred, int idx, uint8_t* out_region) {
+  if (!s || !pred || !out_region) return LTB_FAIL("null argument");
+  if (s->ops.empty()) return LTB_FAIL("this session was created with LTB_SESSION_MEL_ONLY: it has no network");
+  if (idx < 0 || idx >= s->a->n) return LTB_FAIL("paste: idx out of range");
+  if (enter(s)) return 1;
+  std::lock_guard<std::mutex> lk(s->mu);
+  const int* c = &s->a->coords_host[(size_t)idx * 4];
+  LTB_CUDA(cudaMemcpyAsync(s->pred_scratch, pred, (size_t)65536 * 3 * 4, cudaMemcpyHostToDevice, s->st));
+  return region_enqueue_d2h(s, s->pred_scratch, 0, idx, 1, out_region, c[1] - c[0], c[3] - c[2], nullptr);
 }
 
 int ltb_w2l_mel_resident(ltb_w2l_session* s) {
@@ -1168,6 +1257,7 @@ int ltb_w2l_mel_resident(ltb_w2l_session* s) {
 
 int ltb_w2l_step_async(ltb_w2l_session* s, int index) {
   if (!s) return LTB_FAIL("null session");
+  if (need_frames(s->a, "ltb_w2l_step_async")) return 1;
   if (enter(s)) return 1;
   std::lock_guard<std::mutex> lk(s->mu);
   if (forward_enqueue(s, index, true)) return 1;
@@ -1227,6 +1317,7 @@ int ltb_w2l_step_e2e_async(ltb_w2l_session* s, int index, const float* pcm_host,
   if (!s || !pcm_host || !frames_host) return LTB_FAIL("null argument");
   const int expect = (s->l + s->r + 2 * s->B) * 320;
   if (nsamples != expect) return LTB_FAIL("step_e2e: expected " + std::to_string(expect) + " samples");
+  if (need_frames(s->a, "ltb_w2l_step_e2e_async")) return 1;
   if (enter(s)) return 1;
   std::lock_guard<std::mutex> lk(s->mu);
   if (!s->st_copy) {

@@ -21,6 +21,37 @@ def device_count() -> int:
     return n.value
 
 
+def mem_get_info() -> tuple:
+    """(free, total) bytes of the current device (cudaMemGetInfo)."""
+    free, total = C.c_size_t(0), C.c_size_t(0)
+    check(lib().ltb_mem_get_info(C.byref(free), C.byref(total)))
+    return free.value, total.value
+
+
+# Share of the device's free memory (at load time) that an avatar's full frames may take.  Above it an avatar is created
+# frame-free: the frames stay in host RAM, as the reference keeps them, and the device composites only the paste rectangle.
+FRAMES_DEVICE_SHARE = 0.25
+# Frames below this size are uploaded without asking the device: a session's own activation arena is ~0.9 GB, so on a device
+# that can run one at all, 64 MiB of frames cannot decide between the two residencies.
+FRAMES_ALWAYS_RESIDENT_BYTES = 64 << 20
+
+
+def frames_fit_device(frames_nbytes: int) -> bool:
+    """The residency rule of the avatar plugins: True = upload the full frames, False = create the avatar frame-free."""
+    if frames_nbytes <= FRAMES_ALWAYS_RESIDENT_BYTES:
+        return True
+    free, _total = mem_get_info()
+    return frames_nbytes <= FRAMES_DEVICE_SHARE * free
+
+
+def paste_region(frame: np.ndarray, region: np.ndarray, box) -> np.ndarray:
+    """Host half of a frame-free composite: a fresh, writable copy of `frame` with `region` written at box = (y1, y2, x1, x2)."""
+    y1, y2, x1, x2 = (int(v) for v in box)
+    out = np.array(frame, copy=True)
+    out[y1:y2, x1:x2] = region[:y2 - y1, :x2 - x1]
+    return out
+
+
 def _ptr(a: Optional[np.ndarray]):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
@@ -59,23 +90,38 @@ class W2LModel:
 
 
 class W2LAvatar:
-    """Avatar assets resident in HBM (replaces load_avatar's host lists, wav2lip_avatar.py:72-88)."""
+    """Avatar assets resident in HBM (replaces load_avatar's host lists, wav2lip_avatar.py:72-88).
 
-    def __init__(self, faces: Sequence[np.ndarray], frames: Sequence[np.ndarray], coords: Sequence[Sequence[int]]):
+    frames_resident=False: a frame-free avatar.  Only faces and coords go to the device; `frames` stays the caller's host
+    sequence (not copied), and sessions composite only the paste rectangle (the *_region methods), which the host writes into a
+    copy of its own frame (paste_region)."""
+
+    def __init__(self, faces: Sequence[np.ndarray], frames: Sequence[np.ndarray], coords: Sequence[Sequence[int]],
+                 frames_resident: bool = True):
         self.faces = _carr(np.asarray(faces), np.uint8)
-        self.frames = _carr(np.asarray(frames), np.uint8)
         self.coords = _carr(np.asarray(coords), np.int32)
+        self.frames_resident = bool(frames_resident)
         n = self.faces.shape[0]
         if self.faces.shape != (n, 256, 256, 3):
             raise ValueError(f"faces must be (n,256,256,3) uint8, got {self.faces.shape}")
-        if self.frames.ndim != 4 or self.frames.shape[0] != n or self.frames.shape[3] != 3:
-            raise ValueError(f"frames must be (n,H,W,3) uint8, got {self.frames.shape}")
+        if self.frames_resident:
+            self.frames = _carr(np.asarray(frames), np.uint8)
+            shape = self.frames.shape
+        else:
+            self.frames = frames
+            shapes = {np.shape(f) for f in frames}
+            shape = (len(frames), *shapes.pop()) if len(shapes) == 1 else (len(frames), "mixed")
+        if len(shape) != 4 or shape[0] != n or shape[3] != 3:
+            raise ValueError(f"frames must be (n,H,W,3) uint8, got {shape}")
         if self.coords.shape != (n, 4):
             raise ValueError(f"coords must be (n,4), got {self.coords.shape}")
-        self.n, self.H, self.W = n, self.frames.shape[1], self.frames.shape[2]
+        self.n, self.H, self.W = n, shape[1], shape[2]
         self._h = C.c_void_p()
-        check(lib().ltb_w2l_avatar_create(_ptr(self.faces), _ptr(self.frames), _ptr(self.coords), n, self.H, self.W,
-                                          C.byref(self._h)))
+        check(lib().ltb_w2l_avatar_create(_ptr(self.faces), _ptr(self.frames) if self.frames_resident else None, _ptr(self.coords),
+                                          n, self.H, self.W, C.byref(self._h)))
+        rh, rw = C.c_int(0), C.c_int(0)
+        check(lib().ltb_w2l_avatar_region_max(self._h, C.byref(rh), C.byref(rw)))
+        self.region_max = (rh.value, rw.value)
 
     def close(self):
         if self._h:
@@ -87,6 +133,12 @@ class W2LAvatar:
             self.close()
         except Exception:
             pass
+
+
+def mirror_index(size: int, index: int) -> int:
+    """utils/image.py:26-32 — the frame a batch slot composites (as the engine's kernels compute it)."""
+    turn, res = divmod(index, size)
+    return res if turn % 2 == 0 else size - res - 1
 
 
 class PinnedBuffer:
@@ -200,6 +252,55 @@ class W2LSession:
             out = np.empty((n, self.avatar.H, self.avatar.W, 3), np.uint8)
         check(lib().ltb_w2l_infer_slots(self._h, arr, n, _ptr(out)))
         return out
+
+    # --- region forms (frame-free avatars): rectangles + their boxes; engine.paste_region puts one into a frame copy
+    def infer_paste_region(self, index: int, mel: np.ndarray, out: Optional[np.ndarray] = None):
+        """infer_paste for a frame-free avatar: -> (regions uint8 (batch, rh_max, rw_max, 3), boxes int32 (batch, 4)); slot i's
+        rectangle is regions[i, :y2-y1, :x2-x1] of boxes[i] = (y1, y2, x1, x2) of frame mirror_index(n, index + i)."""
+        mel = _carr(mel, np.float32)
+        if mel.size != self.batch * 80 * 16:
+            raise ValueError(f"mel must hold {self.batch}x80x16 values, got shape {mel.shape}")
+        rh, rw = self.avatar.region_max
+        if out is None:
+            out = np.empty((self.batch, rh, rw, 3), np.uint8)
+        check(lib().ltb_w2l_infer_paste_region(self._h, int(index), _ptr(mel), _ptr(out)))
+        n = self.avatar.n
+        boxes = self.avatar.coords[[mirror_index(n, index + i) for i in range(self.batch)]]
+        return out, boxes
+
+    def infer_slots_region(self, requests, out: Optional[np.ndarray] = None):
+        """infer_slots with region output: -> [(region view (h, w, 3), box (y1, y2, x1, x2)), ...], one per request.  Slot avatars
+        may be frame-free and of any frame size; every box must fit this session's avatar's region_max."""
+        n = len(requests)
+        arr = (_capi.W2LSlot * n)()
+        keep = []
+        for i, (av, idx, mel) in enumerate(requests):
+            m = _carr(mel, np.float32)
+            if m.size != 1280:
+                raise ValueError(f"slot {i}: mel window must be (80,16), got {m.shape}")
+            keep.append(m)
+            arr[i].avatar, arr[i].idx, arr[i].mel = av._h, int(idx), m.ctypes.data_as(C.c_void_p)
+        rh, rw = self.avatar.region_max
+        if out is None:
+            out = np.empty((n, rh, rw, 3), np.uint8)
+        check(lib().ltb_w2l_infer_slots_region(self._h, arr, n, _ptr(out)))
+        res = []
+        for i, (av, idx, _m) in enumerate(requests):
+            box = av.coords[int(idx)]
+            res.append((out[i, :box[1] - box[0], :box[3] - box[2]], box))
+        return res
+
+    def paste_pred_region(self, pred: np.ndarray, idx: int):
+        """paste_pred for a frame-free avatar: -> (region uint8 (y2-y1, x2-x1, 3), box (y1, y2, x1, x2)) of frame idx."""
+        pred = _carr(pred, np.float32)
+        if pred.shape != (256, 256, 3):
+            raise ValueError(f"pred must be (256,256,3), got {pred.shape}")
+        if not 0 <= int(idx) < self.avatar.n:
+            raise ValueError(f"idx {idx} out of range")
+        box = self.avatar.coords[int(idx)]
+        out = np.empty((box[1] - box[0], box[3] - box[2], 3), np.uint8)
+        check(lib().ltb_w2l_paste_pred_region(self._h, _ptr(pred), int(idx), _ptr(out)))
+        return out, box
 
     def mel_resident(self) -> None:
         check(lib().ltb_w2l_mel_resident(self._h))

@@ -25,6 +25,8 @@ from typing import Dict, List, Optional, Sequence
 import numpy as np
 
 from . import _capi
+from ._capi import LtbError
+from .engine import mirror_index
 from .ops import ConvWeight, Ctx, DevTensor
 
 KEY_PAD = 64  # cross-attention keys (50 audio tokens) padded to a multiple of 16
@@ -466,12 +468,20 @@ class MuseTalkModel:
 
 class MuseTalkAvatar:
     """Avatar assets resident in HBM (replaces load_avatar's lists, musetalk_avatar.py:69-91): full frames, bbox
-    (x1,y1,x2,y2), mask crop boxes (x_s,y_s,x_e,y_e), 3-channel blend masks and the pre-computed UNet input latents."""
+    (x1,y1,x2,y2), mask crop boxes (x_s,y_s,x_e,y_e), 3-channel blend masks and the pre-computed UNet input latents.
 
-    def __init__(self, ctx: Ctx, frames, masks, coords, crop_boxes, latents):
+    frames_resident=False: a frame-free avatar — instead of the full frames only their crop boxes (the "body crops", packed like the
+    masks) go to the device (``frames`` is None, ``body`` holds them); sessions composite the blended crop box (the *_region methods)
+    and the host writes it into a copy of its own frame (engine.paste_region).  get_image_blending changes nothing outside it."""
+
+    def __init__(self, ctx: Ctx, frames, masks, coords, crop_boxes, latents, frames_resident: bool = True):
         self.ctx = ctx
-        frames = np.ascontiguousarray(np.asarray(frames), np.uint8)
-        self.n, self.H, self.W = frames.shape[0], frames.shape[1], frames.shape[2]
+        self.frames_resident = bool(frames_resident)
+        if self.frames_resident:
+            frames = np.ascontiguousarray(np.asarray(frames), np.uint8)
+            self.n, self.H, self.W = frames.shape[0], frames.shape[1], frames.shape[2]
+        else:
+            self.n, (self.H, self.W) = len(frames), np.shape(frames[0])[:2]
         self.frames_host = frames
         self.coords_host = np.ascontiguousarray(np.asarray(coords), np.int32).reshape(self.n, 4)
         self.crop_host = np.ascontiguousarray(np.asarray(crop_boxes), np.int32).reshape(self.n, 4)
@@ -488,7 +498,11 @@ class MuseTalkAvatar:
             blobs.append(m.reshape(-1))
             o += m.size
         self.masks_host = [np.asarray(m, np.uint8) for m in masks]
-        self.frames = ctx.upload(frames)
+        c = self.crop_host
+        self.region_max = (int((c[:, 3] - c[:, 1]).max()), int((c[:, 2] - c[:, 0]).max()))
+        self.frames = ctx.upload(frames) if self.frames_resident else None
+        self.body = None if self.frames_resident else ctx.upload(np.concatenate(
+            [np.ascontiguousarray(frames[i][ys:ye, xs:xe], np.uint8).reshape(-1) for i, (xs, ys, xe, ye) in enumerate(c)]))
         self.coords = ctx.upload(self.coords_host)
         self.crop = ctx.upload(self.crop_host)
         self.masks = ctx.upload(np.concatenate(blobs))
@@ -499,6 +513,30 @@ class MuseTalkAvatar:
         lat16 = np.zeros((lat.shape[0], lat.shape[2], lat.shape[3], 16), np.float16)
         lat16[..., :8] = lat.transpose(0, 2, 3, 1)
         self.latents = ctx.upload(lat16)
+
+    def box(self, idx: int):
+        """The crop box of frame idx as (y1, y2, x1, x2), the order engine.paste_region takes."""
+        xs, ys, xe, ye = (int(v) for v in self.crop_host[idx])
+        return (ys, ye, xs, xe)
+
+    def paste_op(self, pred: DevTensor, out: DevTensor, slot0: int, index: int, explicit_idx: int, count: int):
+        """The ltb_op_mt_paste descriptor of `count` jobs: full frames into out (count, H, W, 3), or for a frame-free avatar the
+        blended crop boxes into out (count, rh_max, rw_max, 3)."""
+        op = _capi.MtPasteOp()
+        op.coords, op.crop, op.masks, op.mask_off = self.coords.ptr, self.crop.ptr, self.masks.ptr, self.mask_off.ptr
+        if self.frames_resident:
+            op.frames = self.frames.ptr
+        else:
+            op.body, (op.region_h, op.region_w) = self.body.ptr, self.region_max
+        op.pred, op.out = pred.ptr, out.ptr
+        op.nf, op.H, op.W = self.n, self.H, self.W
+        op.index, op.explicit_idx, op.slot0, op.count = index, explicit_idx, slot0, count
+        op.pred_hw = self.lat_hw * 8
+        return op
+
+    def out_shape(self, count: int) -> tuple:
+        """Shape of the paste output of `count` jobs: full frames, or crop boxes packed at region_max for a frame-free avatar."""
+        return (count, self.H, self.W, 3) if self.frames_resident else (count, *self.region_max, 3)
 
 
 class MuseTalkSession:
@@ -526,7 +564,7 @@ class MuseTalkSession:
         self.audio_pe = ctx.alloc((B * KEY_PAD, model.ucfg.cross_attention_dim), np.float16, zero=True)
         self.latents16 = ctx.alloc((B, hw, hw, 16), np.float16, zero=True)
         self.image_u8 = ctx.alloc((B, hw * 8, hw * 8, 3), np.uint8, zero=True)
-        self.frames_out = ctx.alloc((B, avatar.H, avatar.W, 3), np.uint8, zero=True)
+        self.frames_out = ctx.alloc(avatar.out_shape(B), np.uint8, zero=True)
         self.taps = {} if keep_taps else None
         self._paste_ctx = None
         self._audio_host = np.zeros((B, KEY_PAD, model.ucfg.cross_attention_dim), np.float16)
@@ -568,20 +606,15 @@ class MuseTalkSession:
             return None
 
     # ---- MuseReal.paste_back_frame (musetalk_avatar.py:154-164)
-    def _make_paste_op(self, pred: DevTensor, out: DevTensor, slot0: int, index: int, explicit_idx: int, count: int):
-        a = self.avatar
-        op = _capi.MtPasteOp()
-        op.frames, op.coords, op.crop, op.masks, op.mask_off = a.frames.ptr, a.coords.ptr, a.crop.ptr, a.masks.ptr, a.mask_off.ptr
-        op.pred, op.out = pred.ptr, out.ptr
-        op.nf, op.H, op.W = a.n, a.H, a.W
-        op.index, op.explicit_idx, op.slot0, op.count = index, explicit_idx, slot0, count
-        op.pred_hw = a.lat_hw * 8
-        return op
+    def _need_frames(self, what: str):
+        if not self.avatar.frames_resident:
+            raise LtbError(f"{what}: the avatar was created frame-free (frames_resident=False); use the *_region methods")
 
     def _paste_op(self, pred: DevTensor, slot0: int, index: int, explicit_idx: int, count: int):
-        self.ctx.mt_paste(self._make_paste_op(pred, self.frames_out, slot0, index, explicit_idx, count))
+        self.ctx.mt_paste(self.avatar.paste_op(pred, self.frames_out, slot0, index, explicit_idx, count))
 
     def paste(self, slot: int, idx: int) -> np.ndarray:
+        self._need_frames("paste")
         if not (0 <= slot < self.B and 0 <= idx < self.avatar.n):
             raise ValueError("paste: slot / idx out of range")
         with self.ctx.lock:
@@ -592,26 +625,50 @@ class MuseTalkSession:
     def paste_pred(self, pred_u8: np.ndarray, idx: int) -> np.ndarray:
         """paste_back_frame for a host prediction (S,S,3) uint8 — the reference's exact argument.  Runs on its own small
         ctx (stream + scratch prediction + output frame): process_frames calls it while inference_batch is in flight."""
+        self._need_frames("paste_pred")
+        return self._paste_pred(pred_u8, idx, "paste_pred")
+
+    def paste_pred_region(self, pred_u8: np.ndarray, idx: int):
+        """paste_pred for a frame-free avatar: -> (the blended crop box uint8 (y_e-y_s, x_e-x_s, 3), box (y_s, y_e, x_s, x_e))."""
+        if self.avatar.frames_resident:
+            raise LtbError("paste_pred_region: the avatar holds full frames; use paste_pred")
+        region = self._paste_pred(pred_u8, idx, "paste_pred_region")
+        box = self.avatar.box(idx)
+        return region[:box[1] - box[0], :box[3] - box[2]], box
+
+    def _paste_pred(self, pred_u8: np.ndarray, idx: int, what: str) -> np.ndarray:
         S = self.avatar.lat_hw * 8
         pred_u8 = np.ascontiguousarray(pred_u8, np.uint8)
         if pred_u8.shape != (S, S, 3):
-            raise ValueError(f"paste_pred: prediction must be ({S},{S},3) uint8, got {pred_u8.shape}")
+            raise ValueError(f"{what}: prediction must be ({S},{S},3) uint8, got {pred_u8.shape}")
         if not 0 <= idx < self.avatar.n:
-            raise ValueError("paste_pred: idx out of range")
+            raise ValueError(f"{what}: idx out of range")
         if self._paste_ctx is None:
             self._paste_ctx = Ctx()
             self._pred_scratch = self._paste_ctx.alloc((1, S, S, 3), np.uint8)
-            self._paste_out = self._paste_ctx.alloc((self.avatar.H, self.avatar.W, 3), np.uint8)
+            self._paste_out = self._paste_ctx.alloc(self.avatar.out_shape(1)[1:], np.uint8)
         pc = self._paste_ctx
         with pc.lock:
             pc.h2d(self._pred_scratch, pred_u8, sync=False)
-            pc.mt_paste(self._make_paste_op(self._pred_scratch, self._paste_out, 0, 0, idx, 1))
+            pc.mt_paste(self.avatar.paste_op(self._pred_scratch, self._paste_out, 0, 0, idx, 1))
             return pc.download(self._paste_out)
 
     def paste_batch_async(self, index: int):
         self._paste_op(self.image_u8, 0, index, -1, self.B)
 
+    def paste_batch_region(self, index: int, out: Optional[np.ndarray] = None):
+        """paste_batch for a frame-free avatar: -> (regions uint8 (B, rh_max, rw_max, 3), boxes); slot i's blended crop box is
+        regions[i, :y_e-y_s, :x_e-x_s] of frame mirror_index(n, index + i)."""
+        if self.avatar.frames_resident:
+            raise LtbError("paste_batch_region: the avatar holds full frames; use paste_batch")
+        a = self.avatar
+        with self.ctx.lock:
+            self.paste_batch_async(index)
+            regions = self.ctx.download(self.frames_out, out)
+        return regions, [a.box(mirror_index(a.n, index + i)) for i in range(self.B)]
+
     def paste_batch(self, index: int, out: Optional[np.ndarray] = None) -> np.ndarray:
+        self._need_frames("paste_batch")
         with self.ctx.lock:
             self.paste_batch_async(index)
             return self.ctx.download(self.frames_out, out)
@@ -636,6 +693,7 @@ class MuseTalkSession:
 
     def step_async(self, index: int):
         """Everything resident (audio features already on the device): UNet + VAE decode + blend paste-back."""
+        self._need_frames("step_async")
         self.infer_async(index, None)
         self.paste_batch_async(index)
 
@@ -719,24 +777,20 @@ class MuseTalkBatchSession:
     infer_slots = infer_groups
 
     def _out(self, g: int, av: MuseTalkAvatar) -> DevTensor:
-        key = (g, av.H, av.W)
+        shape = av.out_shape(self.Bs)
+        key = (g, *shape)
         if key not in self._frames_out:
-            self._frames_out[key] = self.ctx.alloc((self.Bs, av.H, av.W, 3), np.uint8, zero=True)
+            self._frames_out[key] = self.ctx.alloc(shape, np.uint8, zero=True)
         return self._frames_out[key]
 
     def paste_async(self, requests: Sequence[tuple]) -> List[DevTensor]:
-        """Blend paste-back of every group's predictions into its own avatar frames (device resident; MuseReal.paste_back_frame x Bs)."""
+        """Blend paste-back of every group's predictions into its own avatar frames (device resident; MuseReal.paste_back_frame x Bs).
+        A frame-free avatar's group gets its blended crop boxes instead, (Bs, rh_max, rw_max, 3) (see MuseTalkAvatar.box)."""
         self._check(requests)
         outs = []
         for g, (a, index, _f) in enumerate(requests):
-            op = _capi.MtPasteOp()
-            op.frames, op.coords, op.crop, op.masks, op.mask_off = a.frames.ptr, a.coords.ptr, a.crop.ptr, a.masks.ptr, a.mask_off.ptr
             out = self._out(g, a)
-            op.pred, op.out = self.image_u8.ptr, out.ptr
-            op.nf, op.H, op.W = a.n, a.H, a.W
-            op.index, op.explicit_idx, op.slot0, op.count = int(index), -1, g * self.Bs, self.Bs
-            op.pred_hw = a.lat_hw * 8
-            self.ctx.mt_paste(op)
+            self.ctx.mt_paste(a.paste_op(self.image_u8, out, g * self.Bs, int(index), -1, self.Bs))
             outs.append(out)
         return outs
 
@@ -745,7 +799,8 @@ class MuseTalkBatchSession:
         self.paste_async(requests)
 
     def step(self, requests: Sequence[tuple]) -> List[np.ndarray]:
-        """One batched round: returns, per session, its Bs composited frames (Bs, H, W, 3) uint8."""
+        """One batched round: returns, per session, its Bs composited frames (Bs, H, W, 3) uint8 — for a frame-free avatar its Bs
+        blended crop boxes (Bs, rh_max, rw_max, 3), crop box of frame mirror_index(n, index + i) = MuseTalkAvatar.box."""
         with self.ctx.lock:
             self.infer_async(requests)
             outs = [self.ctx.download(t, sync=False) for t in self.paste_async(requests)]

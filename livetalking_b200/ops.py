@@ -240,6 +240,11 @@ class Ctx:
         check(lib().ltb_op_ul_paste(self._h, C.c_void_p(frames.ptr), C.c_void_p(faces.ptr), C.c_void_p(coords.ptr), C.c_void_p(pred.ptr),
                                     C.c_void_p(out.ptr), nf, H, W, index, explicit_idx, slot0, count))
 
+    def ul_paste_region(self, faces: DevTensor, coords: DevTensor, pred: DevTensor, out: DevTensor, nf: int, rh: int, rw: int, index: int,
+                        explicit_idx: int, slot0: int, count: int):
+        check(lib().ltb_op_ul_paste_region(self._h, C.c_void_p(faces.ptr), C.c_void_p(coords.ptr), C.c_void_p(pred.ptr), C.c_void_p(out.ptr),
+                                           nf, rh, rw, index, explicit_idx, slot0, count))
+
     def hubert_conv0(self, pcm: DevTensor, n: int, w: DevTensor, bias: Optional[DevTensor], Cc: int, stats: DevTensor, out: DevTensor):
         check(lib().ltb_op_hubert_conv0(self._h, C.c_void_p(pcm.ptr), n, C.c_void_p(w.ptr), C.c_void_p(bias.ptr) if bias is not None else None,
                                         Cc, C.c_void_p(stats.ptr), C.c_void_p(out.ptr)))

@@ -5,6 +5,11 @@ and the class registered as ``("avatar", "musetalk")``.  ``MuseReal`` keeps the 
 
     inference_batch(index, audiofeat_batch) -> (B,256,256,3) uint8 BGR predictions      (musetalk_avatar.py:130-152)
     paste_back_frame(pred_frame, idx)       -> H x W x 3 uint8 BGR, fresh and writable   (musetalk_avatar.py:154-164)
+
+Frame-free avatars: the engine avatar gets the full frames only while they fit ``engine.frames_fit_device`` (a fixed share of the
+device's free memory when the avatar is uploaded); otherwise it holds the crop boxes of the frames (what get_image_blending reads),
+the device blends only the crop box, and ``paste_back_frame`` writes it into a fresh copy of ``frame_list_cycle[idx]``.  Single-session
+and cross-session modes work with either residency and hand ``BaseAvatar`` the same frames.
 """
 from __future__ import annotations
 
@@ -43,6 +48,16 @@ class EngineModel:
 
 class AvatarPayload(tuple):
     engine_avatar = None
+    frames_resident = None       # None: the residency rule decides when the engine avatar is created
+
+
+def _engine_avatar(model: EngineModel, lists, frames_resident=None) -> MuseTalkAvatar:
+    frames, masks, coords, mask_coords, latents = lists
+    if frames_resident is None:
+        frames_resident = engine.frames_fit_device(sum(np.asarray(f).nbytes for f in frames))
+    if frames_resident:
+        return MuseTalkAvatar(model.ctx, frames, masks, coords, mask_coords, latents)
+    return MuseTalkAvatar(model.ctx, frames, masks, coords, mask_coords, latents, frames_resident=False)
 
 
 def _load_state_dict(path):
@@ -93,10 +108,12 @@ def load_avatar(avatar_id, model: EngineModel = None):
     return make_avatar(frames, masks, coords, mask_coords, latents, model)
 
 
-def make_avatar(frames, masks, coords, mask_coords, latents, model: EngineModel = None) -> AvatarPayload:
+def make_avatar(frames, masks, coords, mask_coords, latents, model: EngineModel = None, frames_resident=None) -> AvatarPayload:
+    """frames_resident: None = the residency rule (engine.frames_fit_device); False forces a frame-free avatar."""
     payload = AvatarPayload((frames, masks, coords, mask_coords, latents))
+    payload.frames_resident = frames_resident
     if model is not None:
-        payload.engine_avatar = MuseTalkAvatar(model.ctx, frames, masks, coords, mask_coords, latents)
+        payload.engine_avatar = _engine_avatar(model, payload, frames_resident)
     return payload
 
 
@@ -132,11 +149,11 @@ class MuseReal(BaseAvatar):
         if eng_avatar is None:
             # app.py:86-91 calls load_avatar(avatar_id) without the model and shares the payload between sessions: upload once,
             # cache on the payload (a plain tuple from elsewhere cannot carry it and is uploaded per session)
-            eng_avatar = MuseTalkAvatar(model.ctx, self.frame_list_cycle, self.mask_list_cycle, self.coord_list_cycle,
-                                        self.mask_coords_list_cycle, self.input_latent_list_cycle)
+            eng_avatar = _engine_avatar(model, tuple(avatar), getattr(avatar, "frames_resident", None))
             if isinstance(avatar, AvatarPayload):
                 avatar.engine_avatar = eng_avatar
         self._engine_avatar = eng_avatar
+        self._frame_free = not getattr(eng_avatar, "frames_resident", True)
         cross = bool(getattr(opt, "ltb_cross_session", False)) or os.environ.get("LTB_CROSS_SESSION", "0") == "1"
         self._batcher = shared_batcher(model, eng_avatar.lat_hw, self.batch_size) if cross else None
         # every session owns its stream + scratch (two: UNet/VAE graph, Whisper graph); weights / avatar assets are shared.
@@ -166,4 +183,7 @@ class MuseReal(BaseAvatar):
         return self.engine_session.infer(index, whisper_batch)                      # uint8 (B,256,256,3) BGR, as decode_latents
 
     def paste_back_frame(self, pred_frame, idx: int):
+        if self._frame_free:
+            region, box = self.engine_session.paste_pred_region(np.asarray(pred_frame).astype(np.uint8), idx)
+            return engine.paste_region(self.frame_list_cycle[idx], region, box)
         return self.engine_session.paste_pred(np.asarray(pred_frame).astype(np.uint8), idx)

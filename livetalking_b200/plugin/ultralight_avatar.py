@@ -8,7 +8,11 @@ and the class registered as ``("avatar", "ultralight")``.  ``LightReal`` keeps t
 
 Default (fused) mode: ``inference_batch`` runs prep + U-Net + paste-back on the device and returns B ``EngineFrame`` tokens that
 already hold the composited frames; ``paste_back_frame`` hands the matching one out.  ``opt.ltb_return_pred = True`` restores the
-reference's exact data flow (float32 (B,160,160,3) predictions x 255, pasted per frame from the host)."""
+reference's exact data flow (float32 (B,160,160,3) predictions x 255, pasted per frame from the host).
+
+Frame-free avatars: ``make_avatar`` uploads the full frames only while they fit ``engine.frames_fit_device``; otherwise the device
+holds the crops and boxes only, composites just the bbox rectangle, and ``paste_back_frame`` writes it into a fresh copy of
+``frame_list_cycle[idx]``.  Both modes work with either residency and hand ``BaseAvatar`` the same frames."""
 from __future__ import annotations
 
 import glob
@@ -40,6 +44,14 @@ class EngineFrame:
         self.frame, self.idx = frame, idx
 
 
+class EngineRegion:
+    """Frame-free form of EngineFrame: the composited bbox rectangle of frame idx and its box (y1, y2, x1, x2)."""
+    __slots__ = ("region", "box", "idx")
+
+    def __init__(self, region, box, idx):
+        self.region, self.box, self.idx = region, box, idx
+
+
 class EngineAudio:
     """What load_model() returns as ``audio_processor``: the resident HuBERT encoder; sessions build their own extractor graph."""
 
@@ -63,11 +75,17 @@ def load_model(opt=None, hubert_dir="./models/hubert-large-ls960-ft"):
     return make_model(HubertModel.from_pretrained(hubert_dir).state_dict())
 
 
-def make_avatar(unet_sd, frames, faces, coords, ctx: Ctx = None) -> AvatarPayload:
+def make_avatar(unet_sd, frames, faces, coords, ctx: Ctx = None, frames_resident=None) -> AvatarPayload:
+    """frames_resident: None = the residency rule (engine.frames_fit_device); False forces a frame-free avatar."""
+    if frames_resident is None:
+        frames_resident = engine.frames_fit_device(sum(np.asarray(f).nbytes for f in frames))
     ctx = ctx or Ctx()
     net = UltraLightModel(ctx, unet_sd)
     payload = AvatarPayload((net, frames, faces, coords))
-    payload.engine_avatar = UltraLightAvatar(ctx, net, frames, faces, coords)
+    if frames_resident:
+        payload.engine_avatar = UltraLightAvatar(ctx, net, frames, faces, coords)
+    else:
+        payload.engine_avatar = UltraLightAvatar(ctx, net, frames, faces, coords, frames_resident=False)
     return payload
 
 
@@ -103,6 +121,7 @@ class LightReal(BaseAvatar):
         if eng_avatar is None:
             raise RuntimeError("LightReal needs the payload of livetalking_b200.plugin.ultralight_avatar.load_avatar / make_avatar")
         self._engine_avatar = eng_avatar
+        self._frame_free = not getattr(eng_avatar, "frames_resident", True)
         self._return_pred = bool(getattr(opt, "ltb_return_pred", False))
         # every session owns its stream + scratch (two: U-Net graph, HuBERT graph); weights / avatar assets are shared
         self.engine_session = UltraLightSession(eng_avatar, self.batch_size)
@@ -114,7 +133,7 @@ class LightReal(BaseAvatar):
         self._ring, self._ring_pos = [], 0
         if not self._return_pred:
             try:
-                shape = (self.batch_size, eng_avatar.H, eng_avatar.W, 3)
+                shape = (self.batch_size, *(eng_avatar.region_max if self._frame_free else (eng_avatar.H, eng_avatar.W)), 3)
                 self._ring = [engine.PinnedBuffer(shape, np.uint8) for _ in range(max(4, int(os.environ.get("LTB_PIN_RING", "4"))))]
             except Exception as e:   # pinned memory exhausted: pageable output buffers
                 logger.warning("pinned output ring unavailable (%r): using pageable buffers", e)
@@ -158,13 +177,21 @@ class LightReal(BaseAvatar):
         feats = self._features(audiofeat_batch)
         if self._return_pred:
             return self.engine_session.infer(index, feats, want_pred=True)          # float32 (B,160,160,3), as the reference
-        frames = self.engine_session.infer_paste(index, feats, out=self._next_out())   # (B,H,W,3) uint8: one engine round, one D2H
         length = len(self.face_list_cycle)
+        if self._frame_free:
+            regions, boxes = self.engine_session.infer_paste_region(index, feats, out=self._next_out())
+            return [EngineRegion(regions[i], boxes[i], mirror_index(length, index + i)) for i in range(self.batch_size)]
+        frames = self.engine_session.infer_paste(index, feats, out=self._next_out())   # (B,H,W,3) uint8: one engine round, one D2H
         return [EngineFrame(frames[i], mirror_index(length, index + i)) for i in range(self.batch_size)]
 
     def paste_back_frame(self, pred_frame, idx: int):
+        if isinstance(pred_frame, (EngineFrame, EngineRegion)) and pred_frame.idx != idx:
+            raise ValueError(f"paste_back_frame: frame was composited for idx {pred_frame.idx}, asked for {idx}")
         if isinstance(pred_frame, EngineFrame):
-            if pred_frame.idx != idx:
-                raise ValueError(f"paste_back_frame: frame was composited for idx {pred_frame.idx}, asked for {idx}")
             return np.array(pred_frame.frame, copy=True)                              # fresh, writable, owned by Python
+        if isinstance(pred_frame, EngineRegion):
+            return engine.paste_region(self.frame_list_cycle[idx], pred_frame.region, pred_frame.box)
+        if self._frame_free:
+            region, box = self.engine_session.paste_pred_region(np.asarray(pred_frame, dtype=np.float32), idx)
+            return engine.paste_region(self.frame_list_cycle[idx], region, box)
         return self.engine_session.paste_pred(np.asarray(pred_frame, dtype=np.float32), idx)

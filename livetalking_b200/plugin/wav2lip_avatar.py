@@ -12,6 +12,11 @@ base_avatar.py:374-376, 433): the whole batch is composited on the GPU right aft
 once; ``paste_back_frame`` then only hands out the finished frame.  With ``opt.ltb_return_pred = True`` the plugin
 returns the reference's exact data instead (float32 (B,256,256,3) predictions; paste on demand).
 
+Frame-free avatars: ``make_avatar`` uploads the full frames only while they fit ``engine.frames_fit_device`` (a fixed share of
+the device's free memory at load time).  A larger avatar keeps its frames in host RAM, as the reference does; the device then
+composites only the paste rectangle, and ``paste_back_frame`` writes it into a fresh copy of ``frame_list_cycle[idx]``.  Every
+mode below works with either residency and hands ``BaseAvatar`` the same frames.
+
 Cross-session batching (``opt.ltb_cross_session = True`` or ``LTB_CROSS_SESSION=1``): the session owns no network; its
 frames are slot requests to a scheduler shared by all sessions of the model (plugin/batcher.py), which packs up to
 ``LTB_MUX_BATCH`` (16) frames of different sessions into one forward + paste launch.  The session's own ``batch_size`` can
@@ -52,6 +57,24 @@ class EngineFrame:
         self.frame, self.idx = frame, idx
 
 
+class EngineRegion:
+    """Frame-free form of EngineFrame: the composited paste rectangle of frame idx and its box (y1, y2, x1, x2)."""
+    __slots__ = ("region", "box", "idx")
+
+    def __init__(self, region, box, idx):
+        self.region, self.box, self.idx = region, box, idx
+
+
+class _RegionMux:
+    """A slots session of a frame-free avatar as a CrossSessionBatcher mux: one (region, box) per request."""
+
+    def __init__(self, session):
+        self.session, self.batch = session, session.batch
+
+    def infer_slots(self, requests):
+        return self.session.infer_slots_region(requests)
+
+
 def load_model(path):
     """wav2lip_avatar.py:59-70 — checkpoint["state_dict"] (optional 'module.' prefixes) -> resident engine weights."""
     import torch
@@ -77,9 +100,15 @@ def load_avatar(avatar_id):
     return make_avatar(frame_list_cycle, face_list_cycle, coord_list_cycle)
 
 
-def make_avatar(frame_list_cycle, face_list_cycle, coord_list_cycle) -> AvatarPayload:
+def make_avatar(frame_list_cycle, face_list_cycle, coord_list_cycle, frames_resident=None) -> AvatarPayload:
+    """frames_resident: None = the residency rule (engine.frames_fit_device); False forces a frame-free avatar."""
+    if frames_resident is None:
+        frames_resident = engine.frames_fit_device(sum(np.asarray(f).nbytes for f in frame_list_cycle))
     payload = AvatarPayload((frame_list_cycle, face_list_cycle, coord_list_cycle))
-    payload.engine_avatar = engine.W2LAvatar(face_list_cycle, frame_list_cycle, coord_list_cycle)
+    if frames_resident:
+        payload.engine_avatar = engine.W2LAvatar(face_list_cycle, frame_list_cycle, coord_list_cycle)
+    else:
+        payload.engine_avatar = engine.W2LAvatar(face_list_cycle, frame_list_cycle, coord_list_cycle, frames_resident=False)
     return payload
 
 
@@ -92,15 +121,17 @@ _BATCHER_LOCK = __import__("threading").Lock()
 
 
 def shared_batcher(model, eng_avatar) -> CrossSessionBatcher:
-    """One scheduler per (model, frame size): created by the first session that asks, shared by all later ones."""
+    """One scheduler per (model, frame size), or per (model, region capacity) for frame-free avatars: created by the first
+    session that asks, shared by all later ones."""
     with _BATCHER_LOCK:
         table = getattr(model, "_ltb_batchers", None)
         if table is None:
             table = model._ltb_batchers = {}
-        key = (eng_avatar.H, eng_avatar.W)
+        frame_free = not getattr(eng_avatar, "frames_resident", True)
+        key = ("region", *eng_avatar.region_max) if frame_free else (eng_avatar.H, eng_avatar.W)
         if key not in table:
             mux = engine.W2LSession(model, eng_avatar, int(os.environ.get("LTB_MUX_BATCH", "16")), slots=True)
-            table[key] = CrossSessionBatcher(mux, float(os.environ.get("LTB_MUX_WAIT_MS", "4")))
+            table[key] = CrossSessionBatcher(_RegionMux(mux) if frame_free else mux, float(os.environ.get("LTB_MUX_WAIT_MS", "4")))
         return table[key]
 
 
@@ -114,6 +145,7 @@ class LipReal(BaseAvatar):
         if eng_avatar is None:   # a plain tuple from somewhere else: upload now
             eng_avatar = engine.W2LAvatar(self.face_list_cycle, self.frame_list_cycle, self.coord_list_cycle)
         self._engine_avatar = eng_avatar
+        self._frame_free = not getattr(eng_avatar, "frames_resident", True)
         self._return_pred = bool(getattr(opt, "ltb_return_pred", False))
         cross = bool(getattr(opt, "ltb_cross_session", False)) or os.environ.get("LTB_CROSS_SESSION", "0") == "1"
         self._batcher = None
@@ -130,7 +162,7 @@ class LipReal(BaseAvatar):
         # produced and the one being pasted, so 4 is the minimum safe depth.
         self._ring, self._ring_pos = [], 0
         if self._batcher is None and not self._return_pred:
-            shape = (self.batch_size, eng_avatar.H, eng_avatar.W, 3)
+            shape = (self.batch_size, *(eng_avatar.region_max if self._frame_free else (eng_avatar.H, eng_avatar.W)), 3)
             try:
                 self._ring = [engine.PinnedBuffer(shape, np.uint8) for _ in range(max(4, int(os.environ.get("LTB_PIN_RING", "4"))))]
             except Exception as e:   # pinned memory exhausted: fall back to pageable output buffers
@@ -166,15 +198,25 @@ class LipReal(BaseAvatar):
         if self._batcher is not None:
             idxs = [mirror_index(length, index + i) for i in range(self.batch_size)]
             frames = self._batcher.submit([(self._engine_avatar, idxs[i], mel[i]) for i in range(self.batch_size)])
+            if self._frame_free:
+                return [EngineRegion(*frames[i], idxs[i]) for i in range(self.batch_size)]
             return [EngineFrame(frames[i], idxs[i]) for i in range(self.batch_size)]
         if self._return_pred:
             return self.engine_session.infer(index, mel, want_pred=True)        # float32 (B,256,256,3), as the reference
+        if self._frame_free:
+            regions, boxes = self.engine_session.infer_paste_region(index, mel, out=self._next_out())
+            return [EngineRegion(regions[i], boxes[i], mirror_index(length, index + i)) for i in range(self.batch_size)]
         frames = self.engine_session.infer_paste(index, mel, out=self._next_out())   # (B,H,W,3) uint8: one engine call, one D2H
         return [EngineFrame(frames[i], mirror_index(length, index + i)) for i in range(self.batch_size)]
 
     def paste_back_frame(self, pred_frame, idx: int):
+        if isinstance(pred_frame, (EngineFrame, EngineRegion)) and pred_frame.idx != idx:
+            raise ValueError(f"paste_back_frame: frame was composited for idx {pred_frame.idx}, asked for {idx}")
         if isinstance(pred_frame, EngineFrame):
-            if pred_frame.idx != idx:
-                raise ValueError(f"paste_back_frame: frame was composited for idx {pred_frame.idx}, asked for {idx}")
             return np.array(pred_frame.frame, copy=True)                          # fresh, writable, owned by Python
+        if isinstance(pred_frame, EngineRegion):
+            return engine.paste_region(self.frame_list_cycle[idx], pred_frame.region, pred_frame.box)
+        if self._frame_free:
+            region, box = self.engine_session.paste_pred_region(np.asarray(pred_frame, dtype=np.float32), idx)
+            return engine.paste_region(self.frame_list_cycle[idx], region, box)
         return self.engine_session.paste_pred(np.asarray(pred_frame, dtype=np.float32), idx)

@@ -14,6 +14,8 @@ from typing import Dict, List, Optional
 import numpy as np
 
 from .musetalk import Builder, _Replay, _ceil16, _np
+from ._capi import LtbError
+from .engine import mirror_index
 from .ops import ConvWeight, Ctx, DevTensor
 
 CH = [32, 64, 128, 256, 512]          # unet.py:188
@@ -131,20 +133,35 @@ class UltraLightModel:
 
 class UltraLightAvatar:
     """Avatar assets resident in HBM (replaces load_avatar's lists, ultralight_avatar.py:63-82): full frames, 168x168 face crops,
-    bbox (x1,y1,x2,y2) — and, as in the reference, the avatar's OWN network (``ultralight.pth`` lives in the avatar directory)."""
+    bbox (x1,y1,x2,y2) — and, as in the reference, the avatar's OWN network (``ultralight.pth`` lives in the avatar directory).
 
-    def __init__(self, ctx: Ctx, model: UltraLightModel, frames, faces, coords):
-        frames = np.ascontiguousarray(np.asarray(frames), np.uint8)
+    frames_resident=False: a frame-free avatar — crops and boxes only (``frames`` is None); sessions composite the bbox rectangle
+    (the *_region methods) and the host writes it into a copy of its own frame (engine.paste_region)."""
+
+    def __init__(self, ctx: Ctx, model: UltraLightModel, frames, faces, coords, frames_resident: bool = True):
+        self.frames_resident = bool(frames_resident)
+        if self.frames_resident:
+            frames = np.ascontiguousarray(np.asarray(frames), np.uint8)
+            self.n, self.H, self.W = frames.shape[0], frames.shape[1], frames.shape[2]
+        else:
+            self.n, (self.H, self.W) = len(frames), np.shape(frames[0])[:2]
         faces = np.ascontiguousarray(np.asarray(faces), np.uint8)
-        self.n, self.H, self.W = frames.shape[0], frames.shape[1], frames.shape[2]
         if faces.shape != (self.n, CROP, CROP, 3):
             raise ValueError(f"UltraLight face crops must be ({self.n},{CROP},{CROP},3) uint8, got {faces.shape}")
         self.coords_host = np.ascontiguousarray(np.asarray(coords), np.int32).reshape(self.n, 4)
         for x1, y1, x2, y2 in self.coords_host:
             if not (0 <= x1 < x2 <= self.W and 0 <= y1 < y2 <= self.H):
                 raise ValueError("avatar bbox outside the frame")
+        c = self.coords_host
+        self.region_max = (int((c[:, 3] - c[:, 1]).max()), int((c[:, 2] - c[:, 0]).max()))
         self.ctx, self.model = ctx, model
-        self.frames, self.faces, self.coords = ctx.upload(frames), ctx.upload(faces), ctx.upload(self.coords_host)
+        self.frames = ctx.upload(frames) if self.frames_resident else None
+        self.faces, self.coords = ctx.upload(faces), ctx.upload(self.coords_host)
+
+    def box(self, idx: int):
+        """(y1, y2, x1, x2) of frame idx: the order engine.paste_region takes."""
+        x1, y1, x2, y2 = (int(v) for v in self.coords_host[idx])
+        return (y1, y2, x1, x2)
 
 
 class UltraLightSession:
@@ -160,7 +177,8 @@ class UltraLightSession:
         self.audio16 = ctx.alloc((B, 32, 32, 16), np.float16, zero=True)           # NHWC view of audiofeat.reshape(16, 32, 32)
         self.img16 = ctx.alloc((B, FACE, FACE, 16), np.float16, zero=True)
         self.pred = ctx.alloc((B, FACE, FACE, 3), np.float32, zero=True)
-        self.frames_out = ctx.alloc((B, avatar.H, avatar.W, 3), np.uint8, zero=True)
+        out_hw = (avatar.H, avatar.W) if avatar.frames_resident else avatar.region_max
+        self.frames_out = ctx.alloc((B, *out_hw, 3), np.uint8, zero=True)
         self.taps = {} if keep_taps else None
         self._paste_ctx = None
 
@@ -196,8 +214,13 @@ class UltraLightSession:
             return None
 
     # ---- LightReal.paste_back_frame (ultralight_avatar.py:171-184)
+    def _need_frames(self, what: str):
+        if not self.avatar.frames_resident:
+            raise LtbError(f"{what}: the avatar was created frame-free (frames_resident=False); use the *_region methods")
+
     def paste_batch_async(self, index: int):
         a = self.avatar
+        self._need_frames("paste_batch")
         self.ctx.ul_paste(a.frames, a.faces, a.coords, self.pred, self.frames_out, a.n, a.H, a.W, index, -1, 0, self.B)
 
     def paste_batch(self, index: int, out: Optional[np.ndarray] = None) -> np.ndarray:
@@ -207,6 +230,7 @@ class UltraLightSession:
 
     def infer_paste(self, index: int, audio_feats: Optional[np.ndarray] = None, out: Optional[np.ndarray] = None) -> np.ndarray:
         """inference_batch + B x paste_back_frame as one engine round: (B, H, W, 3) uint8 composited frames."""
+        self._need_frames("infer_paste")
         with self.ctx.lock:
             self.infer_async(index, audio_feats)
             self.paste_batch_async(index)
@@ -214,23 +238,54 @@ class UltraLightSession:
 
     def paste_pred(self, pred_frame: np.ndarray, idx: int) -> np.ndarray:
         """paste_back_frame for a host prediction (160,160,3) — the reference's exact argument; own small ctx (process_frames thread)."""
+        self._need_frames("paste_pred")
         a = self.avatar
-        p = np.ascontiguousarray(pred_frame, np.float32)
-        if p.shape != (FACE, FACE, 3):
-            raise ValueError(f"paste_pred: prediction must be ({FACE},{FACE},3), got {p.shape}")
-        if not 0 <= idx < a.n:
-            raise ValueError("paste_pred: idx out of range")
-        if self._paste_ctx is None:
-            self._paste_ctx = Ctx()
-            self._pred_scratch = self._paste_ctx.alloc((1, FACE, FACE, 3), np.float32)
-            self._paste_out = self._paste_ctx.alloc((a.H, a.W, 3), np.uint8)
-        pc = self._paste_ctx
+        pc, p = self._paste_scratch(pred_frame, idx, "paste_pred")
         with pc.lock:
             pc.h2d(self._pred_scratch, p, sync=False)
             pc.ul_paste(a.frames, a.faces, a.coords, self._pred_scratch, self._paste_out, a.n, a.H, a.W, 0, idx, 0, 1)
             return pc.download(self._paste_out)
 
+    def _paste_scratch(self, pred_frame, idx: int, what: str):
+        a = self.avatar
+        p = np.ascontiguousarray(pred_frame, np.float32)
+        if p.shape != (FACE, FACE, 3):
+            raise ValueError(f"{what}: prediction must be ({FACE},{FACE},3), got {p.shape}")
+        if not 0 <= idx < a.n:
+            raise ValueError(f"{what}: idx out of range")
+        if self._paste_ctx is None:
+            self._paste_ctx = Ctx()
+            self._pred_scratch = self._paste_ctx.alloc((1, FACE, FACE, 3), np.float32)
+            self._paste_out = self._paste_ctx.alloc((a.H, a.W, 3) if a.frames_resident else (*a.region_max, 3), np.uint8)
+        return self._paste_ctx, p
+
+    # ---- region forms (frame-free avatars): rectangles + their boxes (y1, y2, x1, x2); engine.paste_region does the host half
+    def infer_paste_region(self, index: int, audio_feats: Optional[np.ndarray] = None, out: Optional[np.ndarray] = None):
+        """infer_paste with region output: -> (regions uint8 (B, rh_max, rw_max, 3), boxes); slot i's rectangle is
+        regions[i, :y2-y1, :x2-x1] of frame mirror_index(n, index + i)."""
+        a = self.avatar
+        rh, rw = a.region_max
+        packed = DevTensor(self.frames_out.ptr, (self.B, rh, rw, 3), np.uint8)     # fits: every box lies inside the frame
+        with self.ctx.lock:
+            self.infer_async(index, audio_feats)
+            self.ctx.ul_paste_region(a.faces, a.coords, self.pred, packed, a.n, rh, rw, index, -1, 0, self.B)
+            regions = self.ctx.download(packed, out)
+        return regions, [a.box(mirror_index(a.n, index + i)) for i in range(self.B)]
+
+    def paste_pred_region(self, pred_frame: np.ndarray, idx: int):
+        """paste_pred with region output: -> (region uint8 (y2-y1, x2-x1, 3), box (y1, y2, x1, x2))."""
+        a = self.avatar
+        pc, p = self._paste_scratch(pred_frame, idx, "paste_pred_region")
+        box = a.box(idx)
+        h, w = box[1] - box[0], box[3] - box[2]
+        region = DevTensor(self._paste_out.ptr, (h, w, 3), np.uint8)
+        with pc.lock:
+            pc.h2d(self._pred_scratch, p, sync=False)
+            pc.ul_paste_region(a.faces, a.coords, self._pred_scratch, region, a.n, h, w, 0, idx, 0, 1)
+            return pc.download(region), box
+
     def step_async(self, index: int):
+        self._need_frames("step_async")
         self.infer_async(index, None)
         self.paste_batch_async(index)
 
